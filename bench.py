@@ -2,7 +2,7 @@
 """bench.py — shared_tree build throughput (Gbp/s) on B200, BASELINE.json's metric.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
-                    [--bases 3100000000] [--repeat-permille 500] [--seed 42]
+                    [--bases 3100000000] [--repeat-permille 500] [--seed 42] [--dump-outputs DIR]
 
 A "step" is one full shared_tree build (pack + canonicalise + hash-cons every level, ids
 final) of the synthetic genome-shaped sequence of BASELINE.json config 3 (`--bases`
@@ -13,6 +13,11 @@ back).  One JSON line on stdout.
 
 --impl reference times the reference's own CPU build (oracle/_ref when it was compiled,
 else the oracle port) on a bounded sample of the same workload.
+
+--dump-outputs DIR writes the tree of the last timed build as DIR/*.npy (see dump_outputs), so that two
+builds of the project can be compared output for output on the same seeded input.  With N > 1 GPUs it is the
+tree rank 0 gathers from one more sharded build of the same input after the timed steps (builds are
+deterministic, so it equals the last timed one).
 """
 from __future__ import annotations
 
@@ -29,6 +34,7 @@ from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the tree may be read-only; nothing is cached in it
 
 DNA = 12
 METRIC = "shared_tree_build_gbp_per_s"
@@ -49,7 +55,15 @@ def parse_args():
     ap.add_argument("--no-pipeline", action="store_true", help="skip sort/serialize/decode/random-access timings")
     ap.add_argument("--option", action="append", default=[], metavar="NAME=VALUE",
                     help="stb_set_option on the build handle (experiments; the defaults are what is reported)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the tree of the last timed build to DIR/*.npy (float64, a seeded sample of the large tables); "
+                         "with N > 1 GPUs, rank 0's gathered tree of one more build of the same input")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU build computed; --impl reference has no such output")
+    return args
 
 
 def workload_config(args, extra=None):
@@ -268,6 +282,51 @@ def sha256_of_device_bytes(t, nbytes):
     return hashlib.sha256(t[:nbytes].cpu().numpy().tobytes()).hexdigest()
 
 
+# ---------------------------------------------------------------------------- --dump-outputs
+DUMP_ROWS = 1 << 20  # rows of leaves.npy and of nodes.npy at most: 16 + 32 MiB in float64
+
+
+def _sample(n: int, k: int, seed):
+    """Sorted positions of `k` rows out of `n` (all of them when n <= k), a fixed function of (n, k, seed)."""
+    import numpy as np
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).choice(n, size=k, replace=False))
+
+
+def dump_outputs(tree, out_dir: Path, seed: int):
+    """What a build hands its caller, as float64 arrays (every value is below 2^53, so each is exact):
+    counts.npy        width, depth, leaf_count, node_count, root pointer
+    layer_counts.npy  nodes per layer, bottom-up
+    leaves.npy        (position, leaf word) rows of the leaf table
+    nodes.npy         (layer, position, left pointer, right pointer) rows of the node layers
+    Tables longer than DUMP_ROWS are sampled at seeded positions: the leaf table as a whole, the node layers
+    with an equal share each so that the short top layers are always complete."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    counts = tree.layer_counts()
+    leaves = tree.leaves()
+    pos = _sample(len(leaves), DUMP_ROWS, [seed, 0])
+    leaf_rows = np.stack([pos.astype(np.float64), leaves[pos].astype(np.float64)], axis=1)
+    assert len(leaves) == 0 or int(leaves[pos].max()) < (1 << 53), "leaf words wider than a float64 mantissa"
+    del leaves
+    node_rows, share = [], DUMP_ROWS // max(1, len(counts))
+    for k in range(len(counts)):
+        layer = tree.layer(k)
+        pos = _sample(len(layer), share, [seed, 1, k])
+        node_rows.append(np.concatenate([np.full((len(pos), 1), k, np.float64), pos[:, None].astype(np.float64),
+                                         layer[pos].astype(np.float64)], axis=1))
+        del layer
+    arrays = {
+        "counts": np.array([tree.width(), tree.depth(), tree.leaf_count(), tree.node_count(), tree.root()], dtype=np.float64),
+        "layer_counts": np.array(counts, dtype=np.float64),
+        "leaves": leaf_rows,
+        "nodes": np.concatenate(node_rows) if node_rows else np.zeros((0, 4), np.float64),
+    }
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 # ---------------------------------------------------------------------------- algorithmic bytes
 def algorithmic_bytes(n0: int, leaf_unique: int, layer_unique: list[int]):
     """Compulsory HBM bytes per kernel class for one build (DESIGN.md §4): streams only;
@@ -344,6 +403,8 @@ def run_b200(args):
     prof = tree.profile_read()
     tree.profile(False)
     launches = pkg.kernel_launches() - launches0
+    if args.dump_outputs:
+        dump_outputs(tree, args.dump_outputs, args.seed)
     ms_per_step = total_ms / args.steps
     bases_used = tree.width() * DNA
     value = bases_used / (ms_per_step * 1e-3) / 1e9
@@ -771,6 +832,8 @@ def run_b200_dist(args, world, rank, local_rank):
     tree = me.gather(stream=stream.cuda_stream)
     parity = None
     if rank == 0:
+        if args.dump_outputs:  # gathered from the build above, which repeats the last timed one on the same input
+            dump_outputs(tree, args.dump_outputs, args.seed)
         gold = golden_record(args)
         parity = {"golden": gold["name"] if gold else None, "leaves": tree.leaf_count(), "layer_counts": tree.layer_counts()}
         nb_pre = tree.bytes()

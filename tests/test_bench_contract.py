@@ -40,6 +40,12 @@ def test_reference_arm_other_ranks_stay_silent():
     assert res.returncode == 0 and res.stdout.strip() == "", (res.stdout, res.stderr[-1000:])
 
 
+def test_rejects_invalid_arguments():
+    for args in (("--steps", "0"), ("--warmup", "-1"), ("--impl", "reference", "--dump-outputs", "out")):
+        res = run_bench(*args)
+        assert res.returncode == 2 and res.stdout == "", (args, res.stderr[-500:])
+
+
 def test_gpu_arm_fails_loudly_without_a_device():
     import torch
     if torch.cuda.is_available():

@@ -1,103 +1,46 @@
-"""CPU: the C restatement against the live, unmodified reference (oracle/_ref/libref.so).
-Skipped where the reference could not be built (no /root/reference and no shipped _ref)."""
-import numpy as np
+"""CPU: the C restatement against what the unmodified reference returned on seeded fuzz inputs
+(tests/golden/reference_fuzz.json, generator: oracle/gen_golden_fuzz.py).  Where the reference can be built
+(oracle/_ref), its live answers are compared with the same records too."""
+import json
+
+import pytest
+
+from conftest import GOLD
+from oracle import gen_golden_fuzz as fuzz
 
 
-def test_leaf_fuzz(oracle, ref):
-    rng = np.random.default_rng(7)
-    for S in range(1, 17):
-        mask = (1 << (4 * S)) - 1
-        for _ in range(300):
-            v = int.from_bytes(rng.bytes(8), "little") & mask
-            assert oracle.leaf_canonical(v, S) == ref.leaf_canonical(v, S)
-            assert oracle.mirrored(v, S) == ref.mirrored(v, S)
-            assert oracle.inverted(v, S) == ref.inverted(v, S)
-            assert oracle.transposed(v, S) == ref.transposed(v, S)
+@pytest.fixture(scope="module")
+def want():
+    return json.loads((GOLD / "reference_fuzz.json").read_text())
 
 
-def test_node_fuzz(oracle, ref):
-    rng = np.random.default_rng(8)
-    null = 0x9FFFFFFF
-
-    def rp():
-        if rng.integers(8) == 0:
-            return null
-        return oracle.pointer(int(rng.integers(5)), int(rng.integers(2)), int(rng.integers(2)), int(rng.integers(4) == 0))
-
-    for _ in range(20000):
-        l, r = rp(), rp()
-        assert oracle.node_canonical(l, r) == ref.node_canonical(l, r)
+@pytest.fixture(scope="module")
+def checkers(oracle):
+    from oracle.pyoracle import Ref, build_ref
+    return [oracle] + ([Ref()] if build_ref() is not None else [])
 
 
-def test_random_trees(oracle, ref):
-    rng = np.random.default_rng(9)
-    for S, n, alphabet in ((12, 5000, 4), (12, 777, 2), (3, 4097, 4), (16, 1000, 16), (7, 2500, 16)):
-        codes = np.array([1, 2, 4, 8, 3, 12, 7, 14, 0, 9, 5, 11, 13, 10, 6, 15], dtype=np.uint64)[:alphabet]
-        nib = codes[rng.integers(0, alphabet, size=(n, S))]
-        leaves = (nib << (4 * np.arange(S, dtype=np.uint64))).sum(axis=1).astype(np.uint64)
-        leaves[n // 2:n // 2 + n // 8] = leaves[:n // 8]  # planted repeat
-        to, tr = oracle.build(leaves, S), ref.build(leaves, S)
-        _, lo = oracle.build_levels(leaves, S)
-        _, lr = ref.build_levels(leaves, S)
-        assert len(lo) == len(lr) and all(np.array_equal(a, b) for a, b in zip(lo, lr))
-        assert to.serialize() == tr.serialize()
-        for k in range(to.depth() - 1):
-            assert np.array_equal(to.layer(k), tr.layer(k))
-            assert np.array_equal(to.histogram(k), tr.histogram(k)), ("histogram", k)  # src/shared_tree.cpp:316
-        assert to.bytes() == tr.bytes() == len(to.serialize())
-        to.sort(); tr.sort()
-        assert to.serialize() == tr.serialize()
-        assert to.bytes() == tr.bytes() == len(to.serialize())
-        back = oracle.deserialize(tr.serialize(), S)  # the reference's stream parsed by the restatement
-        assert back.width() == n and np.array_equal(back.decode(), leaves)
-        assert np.array_equal(to.decode(), leaves) and np.array_equal(tr.decode(), leaves)
-        idx = rng.integers(0, n, 500).astype(np.uint64)
-        assert np.array_equal(to.random_access(idx), tr.random_access(idx))
+def test_leaf_fuzz(checkers, want):
+    for checker in checkers:
+        assert fuzz.leaf_fuzz(checker) == want["leaf_fuzz"], checker.kind
 
 
-def _random_fasta(rng, n_bases, alphabet, width, records, blank_lines):
-    """Valid FASTA text as the reference accepts it (src/fasta_reader.cpp:40-68): a header or a
-    blank line is never followed directly by another one (the reference would parse the second
-    as data and exit on '>'), no '\\r', symbols from its table only, mixed case."""
-    letters = np.frombuffer(alphabet, dtype=np.uint8)
-    body = letters[rng.integers(0, len(letters), n_bases)].copy()
-    lower = rng.integers(0, 2, n_bases).astype(bool)
-    body[lower] = np.char.lower(body[lower].view("S1")).view(np.uint8)
-    body = body.tobytes()
-    cuts = sorted(set(int(c) for c in rng.integers(1, max(2, n_bases), records - 1))) if records > 1 and n_bases > 2 else []
-    pieces, start = [], 0
-    for k, end in enumerate(cuts + [n_bases]):
-        pieces.append(b">record %d some description\n" % k)
-        chunk = body[start:end]
-        lines = [chunk[i:i + width] for i in range(0, len(chunk), width)] or [b""]
-        for j, line in enumerate(lines):
-            pieces.append(line + b"\n")
-            if blank_lines and line and j + 1 < len(lines) and rng.integers(0, 7) == 0:
-                pieces.append(b"\n")  # a blank line between two data lines is skipped like a header
-        start = end
-    text = b"".join(pieces)
-    return text if rng.integers(0, 2) else text.rstrip(b"\n")  # with and without the final newline
+def test_node_fuzz(oracle, checkers, want):
+    for checker in checkers:
+        assert fuzz.node_fuzz(checker, oracle) == want["node_fuzz"], checker.kind
 
 
-def test_fasta_ingest_fuzz(oracle, ref, tmp_path):
-    """Body extraction + packing + whole build from a FILE through the reference's own reader
-    (fasta_reader + read_genome / shared_tree{path}) against the restatement on the same bytes."""
-    rng = np.random.default_rng(10)
-    acgt, iupac = b"ACGT", b"ACGTRYKMSWBDHVN-"
-    cases = [(12, 5000, acgt, 60, 1, False), (12, 70001, acgt, 70, 3, True), (5, 3333, iupac, 50, 4, True), (16, 4096, iupac, 61, 2, False),
-             (1, 257, acgt, 7, 2, True), (13, 999, iupac, 1, 1, False), (12, 11, acgt, 80, 1, False), (12, 12, acgt, 5, 2, True),
-             (8, 40000, acgt, 100000, 1, False), (12, 25, iupac, 3, 5, True)]
-    for k, (S, n_bases, alphabet, width, records, blanks) in enumerate(cases):
-        if n_bases < S:
-            continue  # undefined in the reference (SIGFPE)
-        text = _random_fasta(rng, n_bases, alphabet, width, records, blanks)
-        path = tmp_path / f"case{k}.fa"
-        path.write_bytes(text)
-        want = ref.read_genome(path, S)
-        got = oracle.fasta_to_leaves(text, S)
-        assert len(got) == len(want) and np.array_equal(got, want), (k, S, n_bases, len(got), len(want))
-        if len(want):
-            tr, to = ref.build_file(path, S), oracle.build(got, S)
-            assert to.serialize() == tr.serialize(), (k, "pre-sort stream")
-            to.sort(); tr.sort()
-            assert to.serialize() == tr.serialize(), (k, "post-sort stream")
+def test_random_trees(oracle, checkers, want):
+    for checker in checkers:
+        got = fuzz.random_trees(checker, oracle)
+        for g, w in zip(got, want["random_trees"]):
+            assert g == w, (checker.kind, w["dna_size"], w["n"])  # src/shared_tree.cpp:316 for the histograms
+        assert len(got) == len(want["random_trees"])
+
+
+def test_fasta_ingest_fuzz(checkers, want):
+    for checker in checkers:
+        got = fuzz.fasta_ingest_fuzz(checker)
+        for g, w in zip(got, want["fasta_ingest_fuzz"]):
+            assert g == w, (checker.kind, w["case"])
+        assert len(got) == len(want["fasta_ingest_fuzz"])
