@@ -66,6 +66,41 @@ def cpu_model() -> str:
     return platform.processor()
 
 
+def tree_record(tree, rec: dict, q: int) -> tuple[float, float]:
+    """Adds the tree's fields to rec, in place: shape, sha256 of the leaf table and of every raw node layer,
+    the stream before and after sort() (which this sorts the tree for), and the answers to q seeded queries.
+    rec must already hold "seed" and "dna_size". Works on either checker's tree (oracle.pyoracle._Tree).
+    Returns the seconds sort() and the queries took."""
+    S = rec["dna_size"]
+    rec.update({
+        "width": int(tree.width()), "depth": int(tree.depth()), "leaves": int(tree.leaf_count()),
+        "nodes": int(tree.node_count()), "layer_counts": [int(c) for c in tree.layer_counts()],
+    })
+    rec["pre_leaves_sha256"] = hashlib.sha256(tree.leaves().tobytes()).hexdigest()
+    rec["pre_layer_sha256"] = [hashlib.sha256(tree.layer(k).tobytes()).hexdigest() for k in range(len(rec["layer_counts"]))]
+    pre = tree.serialize()
+    rec["pre_bytes"] = len(pre)
+    rec["pre_sha256"] = hashlib.sha256(pre).hexdigest()
+    del pre
+    t0 = time.perf_counter()
+    tree.sort()
+    sort_s = time.perf_counter() - t0
+    post = tree.serialize()
+    assert tree.bytes() == len(post)
+    rec["post_bytes"] = len(post)
+    rec["post_sha256"] = hashlib.sha256(post).hexdigest()
+    del post
+    rec["bits_per_base"] = 8.0 * rec["post_bytes"] / (rec["width"] * S)
+    idx = query_indices(rec["seed"], q, rec["width"])
+    t0 = time.perf_counter()
+    ans = tree.random_access(idx)
+    ra_s = time.perf_counter() - t0
+    rec["queries"] = q
+    rec["query_answers_sha256"] = hashlib.sha256(np.ascontiguousarray(ans, dtype="<u8").tobytes()).hexdigest()
+    rec["query_first8"] = [f"{int(v):x}" for v in ans[:8]]
+    return sort_s, ra_s
+
+
 def run_case(name: str, ref: Ref, orc: Oracle) -> dict:
     bases, seed, permille, variant, q = CASES[name]
     t0 = time.perf_counter()
@@ -83,34 +118,9 @@ def run_case(name: str, ref: Ref, orc: Oracle) -> dict:
     construct_s = time.perf_counter() - t0
     os.unlink(path)
     print(f"[{name}] reference build {construct_s:.1f} s", flush=True)
-    rec = {
-        "bases": bases, "seed": seed, "repeat_permille": permille, "variant": variant, "dna_size": DNA,
-        "text_sha256": text_sha,
-        "width": int(tree.width()), "depth": int(tree.depth()), "leaves": int(tree.leaf_count()),
-        "nodes": int(tree.node_count()), "layer_counts": [int(c) for c in tree.layer_counts()],
-    }
-    rec["pre_leaves_sha256"] = hashlib.sha256(tree.leaves().tobytes()).hexdigest()
-    rec["pre_layer_sha256"] = [hashlib.sha256(tree.layer(k).tobytes()).hexdigest() for k in range(len(rec["layer_counts"]))]
-    pre = tree.serialize()
-    rec["pre_bytes"] = len(pre)
-    rec["pre_sha256"] = hashlib.sha256(pre).hexdigest()
-    del pre
-    t0 = time.perf_counter()
-    tree.sort()
-    sort_s = time.perf_counter() - t0
-    post = tree.serialize()
-    assert tree.bytes() == len(post)
-    rec["post_bytes"] = len(post)
-    rec["post_sha256"] = hashlib.sha256(post).hexdigest()
-    del post
-    rec["bits_per_base"] = 8.0 * rec["post_bytes"] / (rec["width"] * DNA)
-    idx = query_indices(seed, q, rec["width"])
-    t0 = time.perf_counter()
-    ans = tree.random_access(idx)
-    ra_s = time.perf_counter() - t0
-    rec["queries"] = q
-    rec["query_answers_sha256"] = hashlib.sha256(np.ascontiguousarray(ans, dtype="<u8").tobytes()).hexdigest()
-    rec["query_first8"] = [f"{int(v):x}" for v in ans[:8]]
+    rec = {"bases": bases, "seed": seed, "repeat_permille": permille, "variant": variant, "dna_size": DNA,
+           "text_sha256": text_sha}
+    sort_s, ra_s = tree_record(tree, rec, q)
     rec["reference_timing"] = {
         "construct_s": round(construct_s, 2), "sort_s": round(sort_s, 2), "random_access_s": round(ra_s, 3),
         "gbp_per_s": rec["width"] * DNA / construct_s / 1e9, "threads": 2,

@@ -189,11 +189,17 @@ class Oracle:
         n = self.lib.orc_fasta_body(text, len(text), out)
         return bytes(out[:n])
 
-    def fasta_to_leaves(self, text: bytes, S: int):
-        cap = len(text) // S + 1
+    def fasta_to_leaves(self, text, S: int):
+        """text: bytes, or a contiguous uint8 array (read in place: no copy of a multi-GB text)."""
+        size = len(text)
+        cap = size // S + 1
         out = np.zeros(cap, dtype=np.uint64)
         bad = C.c_int(-1)
-        n = self.lib.orc_fasta_to_leaves(text, len(text), S, out, cap, C.byref(bad))
+        ptr = text
+        if isinstance(text, np.ndarray):  # `text` keeps the array alive during the call
+            assert text.dtype == np.uint8 and text.flags.c_contiguous
+            ptr = C.cast(text.ctypes.data, C.c_char_p)
+        n = self.lib.orc_fasta_to_leaves(ptr, size, S, out, cap, C.byref(bad))
         if n == 0xFFFFFFFFFFFFFFFF:
             raise ValueError(f"unknown symbol {bad.value}")
         return out[:n].copy()

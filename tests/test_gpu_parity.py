@@ -287,49 +287,39 @@ def test_synthetic_tree_parity(stb, oracle):
 
 
 def _synth_record(name):
+    """A record of tests/golden/synth.json (made by the unmodified reference) or of synth_large.json (made by the
+    oracle, at sizes the reference was not run at)."""
     import json
     from conftest import GOLD
-    return json.loads((GOLD / "synth.json").read_text()).get(name)
+    for f in ("synth.json", "synth_large.json"):
+        rec = json.loads((GOLD / f).read_text()).get(name)
+        if rec is not None:
+            return rec
+    return None
 
 
-@pytest.mark.parametrize("name,entry", [("mid_50mbp", "device"), ("mid_50mbp", "host"), ("large_260mbp", "device"),
-                                        ("large_260mbp", "host"), ("config3_3100mbp", "device"), ("config3_3100mbp", "host"),
-                                        ("largeN_260mbp", "device"), ("largeN_260mbp", "host"),
-                                        ("config3N_3100mbp", "device"), ("config3N_3100mbp", "host")])
-def test_synth_reference_golden(stb, name, entry):
-    """BASELINE.json configs 3 / 5 at FULL size against the UNMODIFIED reference: tests/golden/synth.json holds
-    what oracle/_ref produced for the same generated text (oracle/gen_golden_synth.py): per-layer node counts,
-    sha256 of the leaf table and of every raw node layer, of the stream before and after sort_tree
-    (compress.cpp:183-200, src/shared_tree.cpp:488-513) and of the operator[] answers (:268-291)."""
-    import torch
-    rec = _synth_record(name)
-    if rec is None:
-        pytest.skip(f"tests/golden/synth.json has no record {name} (oracle/gen_golden_synth.py {name})")
-    n = rec["bases"]
-    free, _ = torch.cuda.mem_get_info()
-    if free < 14 * n + (4 << 30):
-        pytest.skip("not enough free device memory for this size")
-    buf = torch.empty(n, dtype=torch.uint8, device="cuda")
-    stb.synth_genome(buf, n, seed=rec["seed"], repeat_permille=rec["repeat_permille"])
-    if rec["variant"] == "nruns":  # N runs (1 % of the bases) and soft-masked lower case: a real assembly's shape
-        stb.synth_mask(buf, seed=rec["seed"])
-    tree = stb.SharedTree(12)
-    if entry == "host":  # stb_build_from_body(STB_HOST): the chunked build behind the copy
-        host = torch.empty(n, dtype=torch.uint8, pin_memory=True)
-        host.copy_(buf)
-        torch.cuda.synchronize()
-        tree.build_from_body(host)
-        del host
-    else:
-        tree.build_from_body(buf)
-    del buf
+# Device workspace of a build, per leaf position. Measured on a B200 (1000 W limit) in a fresh process: the
+# device-FASTA build of the 4.5 Gbp text (375 M positions) raised device use by 42.5 GiB. That figure includes
+# the text and its FASTA copy (9.1 GB) and the extracted body (4.5 GB), which leaves about 85 B per position.
+BUILD_BYTES_PER_POSITION = 96
+
+
+def build_memory_bound(rec):
+    """Free device memory a test that holds the text and builds it wants: text bytes + workspace per leaf
+    position (which is what the build's tables follow, whatever the leaf size) + 4 GB."""
+    return rec["bases"] + BUILD_BYTES_PER_POSITION * (rec["bases"] // rec["dna_size"]) + (4 << 30)
+
+
+def check_record(stb, tree, rec, tables=True):
+    """tree (built, not yet sorted) against a synth record: shape, optionally the leaf table and every raw node
+    layer, the stream before and after sort(), and the answers to the record's seeded queries. Sorts the tree."""
     assert tree.width() == rec["width"] and tree.depth() == rec["depth"]
     assert tree.leaf_count() == rec["leaves"] and tree.node_count() == rec["nodes"]
     assert tree.layer_counts() == rec["layer_counts"]
-    if entry == "device":  # every table, word for word
+    if tables:  # every table, word for word
         assert hashlib.sha256(tree.leaves().tobytes()).hexdigest() == rec["pre_leaves_sha256"]
         for k, want in enumerate(rec["pre_layer_sha256"]):
-            assert hashlib.sha256(tree.layer(k).tobytes()).hexdigest() == want, f"node layer {k} differs from the reference's"
+            assert hashlib.sha256(tree.layer(k).tobytes()).hexdigest() == want, f"node layer {k} differs from the record's"
     pre = tree.serialize()
     assert len(pre) == rec["pre_bytes"] and hashlib.sha256(pre).hexdigest() == rec["pre_sha256"]
     del pre
@@ -342,6 +332,50 @@ def test_synth_reference_golden(stb, name, entry):
     ans = tree.random_access(idx)
     assert [f"{int(v):x}" for v in ans[:8]] == rec["query_first8"]
     assert hashlib.sha256(np.ascontiguousarray(ans, dtype="<u8").tobytes()).hexdigest() == rec["query_answers_sha256"]
+
+
+LARGE_CASES = ("beyond4g_4500mbp", "beyond4gN_4500mbp", "ceiling_s1")
+
+
+@pytest.mark.parametrize("name,entry", [("mid_50mbp", "device"), ("mid_50mbp", "host"), ("large_260mbp", "device"),
+                                        ("large_260mbp", "host"), ("config3_3100mbp", "device"), ("config3_3100mbp", "host"),
+                                        ("largeN_260mbp", "device"), ("largeN_260mbp", "host"),
+                                        ("config3N_3100mbp", "device"), ("config3N_3100mbp", "host")] +
+                         [(name, entry) for name in LARGE_CASES for entry in ("device", "host")])
+def test_synth_reference_golden(stb, name, entry):
+    """Full-size synthetic genomes against records of the same generated text: per-layer node counts, sha256 of the
+    leaf table and of every raw node layer, of the stream before and after sort_tree (compress.cpp:183-200,
+    src/shared_tree.cpp:488-513) and of the operator[] answers (:268-291).
+    tests/golden/synth.json (BASELINE.json configs 3 / 5, up to 3.1 Gbp) was written by the UNMODIFIED reference
+    (oracle/gen_golden_synth.py). tests/golden/synth_large.json was written by the oracle (oracle/gen_golden_large.py,
+    "made_by": "oracle.c"): 4.5 Gbp at dna_size 12, past 2^32 text bytes, plain and with N runs, and 2^30 - 1 bases
+    at dna_size 1, the largest input the build accepts. tests/test_golden_large_host.py checks that the oracle path
+    reproduces the reference's records."""
+    import torch
+    rec = _synth_record(name)
+    if rec is None:
+        pytest.skip(f"tests/golden has no synth record {name} (oracle/gen_golden_synth.py, oracle/gen_golden_large.py)")
+    n, S = rec["bases"], rec["dna_size"]
+    free, _ = torch.cuda.mem_get_info()
+    if free < build_memory_bound(rec):
+        pytest.skip("not enough free device memory for this size")
+    buf = torch.empty(n, dtype=torch.uint8, device="cuda")
+    stb.synth_genome(buf, n, seed=rec["seed"], repeat_permille=rec["repeat_permille"])
+    if rec["variant"] == "nruns":  # N runs (1 % of the bases) and soft-masked lower case: a real assembly's shape
+        stb.synth_mask(buf, seed=rec["seed"])
+    tree = stb.SharedTree(S)
+    if entry == "host":  # stb_build_from_body(STB_HOST): the chunked build behind the copy
+        host = torch.empty(n, dtype=torch.uint8, pin_memory=True)
+        host.copy_(buf)
+        torch.cuda.synchronize()
+        del buf
+        tree.build_from_body(host)
+        del host
+    else:
+        tree.build_from_body(buf)
+        del buf
+    check_record(stb, tree, rec, tables=entry == "device")
+    tree.close()
 
 
 def test_large_properties(stb):
