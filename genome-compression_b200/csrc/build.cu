@@ -523,28 +523,52 @@ struct LeafInput {
   const unsigned long long* leaves = nullptr; // device
 };
 
+// Node tables: a slot's last word is an epoch tag; every node level of every build on this
+// handle takes a fresh serial and sees the slots of earlier levels as empty, so the table is
+// cleared only when its memory is new (or when the serials come near wrapping).
+struct EpochTable {
+  DevBuf<Slot> buf;
+  bool cleared = false;
+  uint32_t serial = 0;
+
+  cudaError_t ensure(uint64_t slots, cudaStream_t st) {
+    bool grew = false;
+    const cudaError_t e = buf.ensure(slots, st, &grew);
+    if (grew) cleared = false;
+    return e;
+  }
+  int clear_if_needed(Ctx& ctx) {
+    if (serial > 0xfff00000u) cleared = false;  // far from wrapping into a tag that is still in the table
+    if (cleared) return STB_OK;
+    Launch l(ctx, "table_clear", false);
+    STB_CUDA(ctx, cudaMemsetAsync(buf.ptr, 0xff, buf.bytes(), ctx.stream));
+    cleared = true;
+    serial = 0;
+    return STB_OK;
+  }
+  uint32_t take(uint32_t k) {  // the first of k fresh serials
+    serial += k;
+    return serial - k + 1;
+  }
+};
+
 struct Scratch {
   DevBuf<uint32_t> ptr_a, ptr_b, aux, bitmask, counts, dminpos, dids;
   DevBuf<uint32_t> lvl_bits[2], lvl_multi[2];  // node levels: first occurrences / first occurrences that occur again, by level parity
   DevBuf<uint32_t> tilecnt;                    // first occurrences per tile, then per chunk of tiles (count_kernel)
-  DevBuf<Slot> slots, side_slots;
+  DevBuf<Slot> side_slots;
   DevBuf<BuildFlags> flags;
   DevBuf<uint32_t> root;
   BucketWorkspace bucket;
-  // Node tables: a slot's last word is an epoch tag; every node level of every build on this
-  // handle takes a fresh serial, so the table is cleared only when its memory is new.
-  bool tags_cleared = false;
-  uint32_t serial = 0;
-  // the streaming build's per-level tables (stream_slots) count their own epochs: a reset of one
-  // counter must never make a tag that is still stored in the other table current again
-  bool stream_tags_cleared = false;
-  uint32_t stream_serial = 0;
+  // The node levels' table (the hashed leaf level uses it untagged), and the streaming build's
+  // per-level tables.  They count their own epochs: a reset of one counter must never make a tag
+  // that is still stored in the other table current again.
+  EpochTable slots, stream_slots;
 
   // streaming build (host input): every chunked level keeps its own pointer array, bitmap,
   // table for the whole build, and a running total per level (two copies: a launch reads one
   // while its last tile writes the other)
   DevBuf<uint32_t> ptr_arena, bit_arena, level_sizes, run_totals;
-  DevBuf<Slot> stream_slots;
   cudaStream_t copy_stream = nullptr;
   std::vector<cudaEvent_t> chunk_events;
   DevBuf<char> stream_body;  // streaming FASTA ingest: the extracted body
@@ -558,16 +582,7 @@ struct Scratch {
 
 Scratch& workspace_of(Tree& t) {
   if (!t.workspace) t.workspace = std::make_shared<Scratch>();
-  Scratch& sc = *static_cast<Scratch*>(t.workspace.get());
-  if (sc.serial > 0xfff00000u) {  // far from wrapping into a tag that is still in the table
-    sc.serial = 0;
-    sc.tags_cleared = false;
-  }
-  if (sc.stream_serial > 0xfff00000u) {
-    sc.stream_serial = 0;
-    sc.stream_tags_cleared = false;
-  }
-  return sc;
+  return *static_cast<Scratch*>(t.workspace.get());
 }
 
 // slots of the side table for leaves outside ACGT next to the direct table (side_insert)
@@ -578,40 +593,63 @@ uint32_t side_table_cap(const Tree& t, uint64_t n0) {
 uint32_t table_cap(uint64_t n) { return (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1024, 2 * n), 0x1ffffffeull); }
 uint64_t bitmap_words(uint64_t n) { return ceil_div(n, LVL_TILE) * (LVL_TILE / 32); }
 
-template <int S_T, bool DIRECT>
-void launch_leaf_text(Ctx& ctx, const char* body, uint64_t n, LevelTable tab, uint32_t* tmp, BuildFlags* flags, uint32_t pos0 = 0) {
+// The leaf level from ASCII text.  ACGT leaves of length 12 next to the direct table take the SWAR kernel.
+void launch_leaf_text(Ctx& ctx, bool direct, const char* body, uint64_t n, LevelTable tab, uint32_t* tmp, BuildFlags* flags, uint32_t pos0 = 0) {
+  const unsigned grid = (unsigned)ceil_div(n, PACK_TILE_LEAVES);
   const size_t smem = pack_smem_bytes(ctx.S);
   Launch l(ctx, "leaf_insert");
-  if (S_T == 12 && DIRECT) {
-    leaf_insert_acgt12_kernel<<<(unsigned)ceil_div(n, PACK_TILE_LEAVES), PACK_THREADS, smem, ctx.stream>>>(body, n, tab, tmp, flags, pos0);
-    return;
-  }
-  leaf_insert_text_kernel<S_T, DIRECT><<<(unsigned)ceil_div(n, PACK_TILE_LEAVES), PACK_THREADS, smem, ctx.stream>>>(
-      body, n, ctx.S, tab, tmp, flags, pos0);
+  if (ctx.S == 12 && direct) leaf_insert_acgt12_kernel<<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, tab, tmp, flags, pos0);
+  else if (ctx.S == 12) leaf_insert_text_kernel<12, false><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, ctx.S, tab, tmp, flags, pos0);
+  else if (direct) leaf_insert_text_kernel<0, true><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, ctx.S, tab, tmp, flags, pos0);
+  else leaf_insert_text_kernel<0, false><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, ctx.S, tab, tmp, flags, pos0);
 }
 
-// assign -> resolve for one level whose inserts are already queued.  `aux` is what the inserts
-// left per position, `out` receives the finished pointers (the same array for the leaf level).
+const BuildFlags NO_FLAGS{~0ull, 0u, 0u, 0u, 0u};
+
+int reset_flags(Ctx& ctx, BuildFlags* flags) {
+  STB_CUDA(ctx, cudaMemcpyAsync(flags, &NO_FLAGS, sizeof(NO_FLAGS), cudaMemcpyHostToDevice, ctx.stream));
+  return STB_OK;
+}
+
+// The input errors the leaf kernels report (non_acgt is not one: the caller decides what it means).
+int check_flags(const Ctx& ctx, const BuildFlags& flags) {
+  if (flags.bad_symbol != ~0ull) return ctx.fail(STB_ERR_UNKNOWN_SYMBOL, unknown_symbol_message((int)(flags.bad_symbol & 0xff)));
+  if (flags.bad_leaf) return ctx.fail(STB_ERR_BAD_LEAF, "packed leaf has bits set at or above 4*dna_size");
+  return STB_OK;
+}
+
+// Tiles [first, first + count) of a level.  `carry` (null: 0) is the level's number of first
+// occurrences before them, `total` receives the number up to their end.
+struct TileWindow {
+  uint32_t first, count;
+  const uint32_t* carry;
+  uint32_t* total;
+};
+TileWindow whole_level(uint64_t n, uint32_t* total) { return {0u, (uint32_t)ceil_div(n, LVL_TILE), nullptr, total}; }
+
+// count -> assign -> resolve over a window of one level whose inserts are already queued.  `aux` is
+// what the inserts left per position, `out` receives the finished pointers (the same array for the
+// leaf level); assign and resolve see positions below n_assign and n_resolve.
 template <int MODE>
-int finish_level(Ctx& ctx, const uint32_t* aux, uint32_t* out, uint32_t n, LevelTable tab, const uint32_t* bitmask, uint32_t* tilecnt,
-                 uint32_t* total_out, void* uniq, const uint32_t* children = nullptr, uint32_t n_children = 0, uint32_t* multi_bits = nullptr,
-                 const uint32_t* firstpos_unless = nullptr, bool skip_resolve = false) {
-  const unsigned nb = (unsigned)ceil_div(n, LVL_TILE);
-  uint32_t* chunkcnt = tilecnt + nb;
-  STB_CUDA(ctx, cudaMemsetAsync(chunkcnt, 0, (nb / CHUNK_TILES + 1) * 4, ctx.stream));
+int finish_level(Ctx& ctx, const TileWindow& w, const uint32_t* aux, uint32_t* out, uint32_t n_assign, uint32_t n_resolve, LevelTable tab,
+                 const uint32_t* bitmask, uint32_t* tilecnt, void* uniq, const uint32_t* children = nullptr, uint32_t n_children = 0,
+                 uint32_t* multi_bits = nullptr, const uint32_t* firstpos_unless = nullptr, bool skip_resolve = false) {
+  uint32_t* chunkcnt = tilecnt + w.count;
+  STB_CUDA(ctx, cudaMemsetAsync(chunkcnt, 0, (w.count / CHUNK_TILES + 1) * 4, ctx.stream));
   {
     Launch l(ctx, "count_firsts");
-    count_kernel<<<(unsigned)ceil_div((uint64_t)nb * 32, 256), 256, 0, ctx.stream>>>(bitmask, 0u, nb, tilecnt, chunkcnt);
+    count_kernel<<<(unsigned)ceil_div((uint64_t)w.count * 32, 256), 256, 0, ctx.stream>>>(bitmask, w.first, w.count, tilecnt, chunkcnt);
   }
   {
     Launch l(ctx, "assign_ids");
-    assign_kernel<MODE><<<nb, LVL_THREADS, 0, ctx.stream>>>(out, n, tab, bitmask, tilecnt, chunkcnt, 0u, nullptr, total_out, uniq, ctx.S, children,
-                                                            n_children);
+    assign_kernel<MODE><<<w.count, LVL_THREADS, 0, ctx.stream>>>(out, n_assign, tab, bitmask, tilecnt, chunkcnt, w.first, w.carry, w.total, uniq, ctx.S,
+                                                                 children, n_children);
   }
   if (!skip_resolve) {
     Launch l(ctx, "resolve_ids");
-    if (MODE == MODE_LEAF_DIRECT) resolve_kernel<RESOLVE_DIRECT><<<nb, LVL_THREADS, 0, ctx.stream>>>(aux, out, n, tab, bitmask, 0u, nullptr, nullptr);
-    else resolve_kernel<RESOLVE_TABLE><<<nb, LVL_THREADS, 0, ctx.stream>>>(aux, out, n, tab, bitmask, 0u, multi_bits, firstpos_unless);
+    if (MODE == MODE_LEAF_DIRECT)
+      resolve_kernel<RESOLVE_DIRECT><<<w.count, LVL_THREADS, 0, ctx.stream>>>(aux, out, n_resolve, tab, bitmask, w.first, multi_bits, firstpos_unless);
+    else resolve_kernel<RESOLVE_TABLE><<<w.count, LVL_THREADS, 0, ctx.stream>>>(aux, out, n_resolve, tab, bitmask, w.first, multi_bits, firstpos_unless);
   }
   return STB_OK;
 }
@@ -633,11 +671,7 @@ int reserve_node_workspace(Tree& t, Scratch& sc, uint64_t n_cur) {
   }
   STB_CUDA(t, sc.counts.ensure(80, st));
   STB_CUDA(t, sc.root.ensure(1, st));
-  {
-    bool grew = false;
-    STB_CUDA(t, sc.slots.ensure((uint64_t)table_cap(n1) + 1, st, &grew));
-    if (grew) sc.tags_cleared = false;
-  }
+  STB_CUDA(t, sc.slots.ensure((uint64_t)table_cap(n1) + 1, st));
   if (n1 >= t.opt.bucket_min && t.opt.bucket_levels > 0) {
     const BucketPlan pl = bucket_plan(n1, t.opt);  // the largest level: later ones fit in what it reserves
     if (pl.usable) STB_TRY(bucket_reserve(t, sc.bucket, pl));
@@ -655,18 +689,11 @@ BucketPlan level_bucket_plan(const Tree& t, uint64_t n_next, int level) {
 // holds the root pointer in *root_buf.  The workspace must have been reserved for n_cur.
 // `leaf` (optional): `cur` holds leaf words whose later occurrences are still unresolved; the first level is then
 // bucketed (the caller checked level_bucket_plan) and its partition pass finishes them (LeafFinish).
-int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t n_cur, uint32_t* counts_dev, int* levels_out,
-                    uint32_t** root_buf, const LeafFinish* leaf = nullptr) {
+int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t n_cur, uint32_t* counts_dev, uint32_t** root_buf,
+                    const LeafFinish* leaf = nullptr) {
   cudaStream_t st = t.stream;
   int level = 0;
-  if (!sc.tags_cleared) {
-    // Node tables are never cleared between levels: a slot's last word is an epoch tag and a
-    // slot whose tag is not this level's serial counts as empty.  One clear per allocation.
-    Launch l(t, "table_clear", false);
-    STB_CUDA(t, cudaMemsetAsync(sc.slots.ptr, 0xff, sc.slots.bytes(), st));
-    sc.tags_cleared = true;
-    sc.serial = 0;
-  }
+  STB_TRY(sc.slots.clear_if_needed(t));  // never cleared between levels (EpochTable)
   const int level_tag0 = t.profile_level;  // the caller's level of `cur` (leaf pointers: 0), or -1
   do {
     if (level_tag0 >= 0) t.profile_level = level_tag0 + level + 1;
@@ -707,10 +734,9 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
       const uint64_t n_first = ceil_div(n_cur, 2);
       STB_CUDA(t, cudaMemsetAsync(sc.lvl_bits[par].ptr, 0, bitmap_words(n_first) * 4, st));
       STB_CUDA(t, cudaMemsetAsync(sc.lvl_multi[par].ptr, 0, bitmap_words(n_first) * 4, st));
-      uint32_t n_cur32 = (uint32_t)n_cur, serial0 = sc.serial + 1, parity = par;
-      sc.serial += (uint32_t)out.levels;
+      uint32_t n_cur32 = (uint32_t)n_cur, serial0 = sc.slots.take((uint32_t)out.levels), parity = par;
       bool first_is_upper = level > 0, use_filter = t.opt.child_filter != 0, locality = t.opt.locality != 0;
-      Slot* slots = sc.slots.ptr;
+      Slot* slots = sc.slots.buf.ptr;
       uint32_t *aux = sc.aux.ptr, *b0 = sc.lvl_bits[0].ptr, *b1 = sc.lvl_bits[1].ptr, *m0 = sc.lvl_multi[0].ptr, *m1 = sc.lvl_multi[1].ptr;
       uint32_t *blockcnt = sc.tilecnt.ptr, *counts = counts_dev + level;
       uint32_t chunk_off = (uint32_t)ceil_div(n_first, LVL_TILE);
@@ -730,7 +756,7 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
     STB_CUDA(t, layer.nodes.alloc(n_next, st));
     uint32_t* first_bits = sc.lvl_bits[par].ptr;
     uint32_t* multi_bits = sc.lvl_multi[par].ptr;
-    LevelTable nt{sc.slots.ptr, nullptr, nullptr, table_cap(n_next)};
+    LevelTable nt{sc.slots.buf.ptr, nullptr, nullptr, table_cap(n_next)};
     nt.first_bits = first_bits;
     STB_CUDA(t, cudaMemsetAsync(first_bits, 0, bitmap_words(n_next) * 4, st));
     STB_CUDA(t, cudaMemsetAsync(multi_bits, 0, bitmap_words(n_next) * 4, st));
@@ -755,53 +781,53 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
       // and chunking the level to keep table lines in L2 did not pay (profiles/README.md).
       Launch l(t, pl.usable ? "bucket_fallback" : "node_insert");
       node_insert_kernel<<<pl.usable ? std::min(nb, 1184u) : nb, LVL_THREADS, 0, st>>>(cur, (uint32_t)n_cur, (uint32_t)n_next, nt, sc.aux.ptr, child_unique,
-                                                                                        ++sc.serial, child_first, child_multi, 0u, overflow);
+                                                                                        sc.slots.take(1), child_first, child_multi, 0u, overflow);
     }
-    STB_TRY(finish_level<MODE_NODE>(t, sc.aux.ptr, nxt, (uint32_t)n_next, nt, first_bits, sc.tilecnt.ptr, counts_dev + level, layer.nodes.ptr, cur,
-                                    (uint32_t)n_cur, multi_bits, overflow));
+    STB_TRY(finish_level<MODE_NODE>(t, whole_level(n_next, counts_dev + level), sc.aux.ptr, nxt, (uint32_t)n_next, (uint32_t)n_next, nt, first_bits,
+                                    sc.tilecnt.ptr, layer.nodes.ptr, cur, (uint32_t)n_cur, multi_bits, overflow));
     std::swap(cur, nxt);
     n_cur = n_next;
     ++level;
   } while (n_cur > 1);
   t.profile_level = level_tag0;
-  *levels_out = level;
   *root_buf = cur;
   return STB_OK;
 }
 
-// Reads back the per-layer counts, the flags and the root; fills in the tree; trims storage.
-int finish_build(Tree& t, Scratch& sc, uint64_t n0, int level, const uint32_t* cur, bool direct) {
+// Copies the item counts at counts_dev (the leaves' first when `leaves`, then one per layer of
+// t.layers) and the root pointer at root_dev to the host, with the build flags when `flags_dev` is
+// given, and waits.  The flags are reported first, then a count at the index ceiling; the tree is
+// cleared when either fails.  Otherwise fills in the counts and the root.
+int read_back(Tree& t, const uint32_t* counts_dev, bool leaves, const uint32_t* root_dev, const BuildFlags* flags_dev = nullptr) {
   cudaStream_t st = t.stream;
-  std::vector<uint32_t> counts(level + 1);
-  BuildFlags flags{};
+  const size_t first_layer = leaves ? 1 : 0;  // index of t.layers[0]'s count
+  std::vector<uint32_t> counts(first_layer + t.layers.size());
+  BuildFlags flags = NO_FLAGS;
   uint32_t root = PTR_NULL;
-  STB_CUDA(t, cudaMemcpyAsync(counts.data(), sc.counts.ptr, counts.size() * 4, cudaMemcpyDeviceToHost, st));
-  STB_CUDA(t, cudaMemcpyAsync(&flags, sc.flags.ptr, sizeof(flags), cudaMemcpyDeviceToHost, st));
-  STB_CUDA(t, cudaMemcpyAsync(&root, cur, 4, cudaMemcpyDeviceToHost, st));
+  STB_CUDA(t, cudaMemcpyAsync(counts.data(), counts_dev, counts.size() * 4, cudaMemcpyDeviceToHost, st));
+  if (flags_dev) STB_CUDA(t, cudaMemcpyAsync(&flags, flags_dev, sizeof(flags), cudaMemcpyDeviceToHost, st));
+  STB_CUDA(t, cudaMemcpyAsync(&root, root_dev, 4, cudaMemcpyDeviceToHost, st));
   STB_CUDA(t, cudaStreamSynchronize(st));
   STB_CUDA(t, cudaGetLastError());
 
-  if (flags.bad_symbol != ~0ull) {
-    t.clear();
-    return t.fail(STB_ERR_UNKNOWN_SYMBOL, unknown_symbol_message((int)(flags.bad_symbol & 0xff)));
-  }
-  if (flags.bad_leaf) {
-    t.clear();
-    return t.fail(STB_ERR_BAD_LEAF, "packed leaf has bits set at or above 4*dna_size");
-  }
-  if (direct && flags.non_acgt) {
-    t.clear();
-    return -1;  // caller retries with the hash-table leaf level
-  }
+  int s = check_flags(t, flags);
+  if (s == STB_OK && flags.non_acgt) s = NOT_APPLICABLE;  // only the direct leaf level raises it: the input needs the hash-table one
   for (uint32_t c : counts)
-    if (c >= IDX_MASK) {
-      t.clear();
-      return t.fail(STB_ERR_INDEX_CEILING, "a layer has 2^29-1 or more unique items; the pointer format cannot index it");
-    }
-
-  t.n_leaves = counts[0];
-  for (int k = 0; k < level; ++k) t.layers[k].count = counts[k + 1];
+    if (s == STB_OK && c >= IDX_MASK) s = t.fail(STB_ERR_INDEX_CEILING, "a layer has 2^29-1 or more unique items; the pointer format cannot index it");
+  if (s != STB_OK) {
+    t.clear();
+    return s;
+  }
+  if (leaves) t.n_leaves = counts[0];
+  for (size_t k = 0; k < t.layers.size(); ++k) t.layers[k].count = counts[first_layer + k];
   t.root = root;
+  return STB_OK;
+}
+
+// Reads back the counts, the flags and the root of a build from leaves; trims storage.
+int finish_build(Tree& t, Scratch& sc, uint64_t n0, const uint32_t* cur) {
+  cudaStream_t st = t.stream;
+  STB_TRY(read_back(t, sc.counts.ptr, true, cur, sc.flags.ptr));
   t.width = n0;
   t.built = true;
   t.plan_valid = false;
@@ -835,23 +861,16 @@ int build_impl(Tree& t, const LeafInput& in, uint64_t n0, bool direct) {
   STB_TRY(reserve_node_workspace(t, sc, n0));
   STB_CUDA(t, sc.bitmask.ensure(bitmap_words(n0), st));
   STB_CUDA(t, sc.flags.ensure(1, st));
-  {
-    BuildFlags init{~0ull, 0u, 0u, 0u, 0u};
-    STB_CUDA(t, cudaMemcpyAsync(sc.flags.ptr, &init, sizeof(init), cudaMemcpyHostToDevice, st));
-  }
+  STB_TRY(reset_flags(t, sc.flags.ptr));
 
   // ---- leaf level ----
   t.profile_level = t.opt.profile_levels ? 0 : -1;
   const uint64_t direct_entries = direct ? (1ull << (2 * S)) : 0;
   const uint32_t leaf_cap = direct ? 0u : table_cap(n0);
-  if (!direct) {
-    bool grew = false;
-    // the hashed leaf level uses the node table untagged: what it leaves there carries the tag
-    // 0xffffffff, which is never a level's serial, so the node levels see those slots as empty
-    STB_CUDA(t, sc.slots.ensure((uint64_t)leaf_cap + 1, st, &grew));
-    if (grew) sc.tags_cleared = false;
-  }
-  LevelTable tab{sc.slots.ptr, nullptr, nullptr, leaf_cap};
+  // the hashed leaf level uses the node table untagged: what it leaves there carries the tag
+  // 0xffffffff, which is never a level's serial, so the node levels see those slots as empty
+  if (!direct) STB_CUDA(t, sc.slots.ensure((uint64_t)leaf_cap + 1, st));
+  LevelTable tab{sc.slots.buf.ptr, nullptr, nullptr, leaf_cap};
   tab.first_bits = sc.bitmask.ptr;
   STB_CUDA(t, cudaMemsetAsync(sc.bitmask.ptr, 0, bitmap_words(n0) * 4, st));
   if (direct) {
@@ -867,19 +886,13 @@ int build_impl(Tree& t, const LeafInput& in, uint64_t n0, bool direct) {
     STB_CUDA(t, cudaMemsetAsync(sc.side_slots.ptr, 0xff, ((uint64_t)tab.cap + 1) * sizeof(Slot), st));
   } else {
     Launch l(t, "table_clear", false);
-    STB_CUDA(t, cudaMemsetAsync(sc.slots.ptr, 0xff, ((uint64_t)leaf_cap + 1) * sizeof(Slot), st));
+    STB_CUDA(t, cudaMemsetAsync(sc.slots.buf.ptr, 0xff, ((uint64_t)leaf_cap + 1) * sizeof(Slot), st));
   }
   const uint64_t leaf_store = direct ? std::min<uint64_t>(n0, direct_entries / 2 + side_table_cap(t, n0) / 2 + 2) : n0;
   STB_CUDA(t, t.leaves.alloc(leaf_store, st));
 
   if (in.body) {
-    if (direct) {
-      if (S == 12) launch_leaf_text<12, true>(t, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
-      else launch_leaf_text<0, true>(t, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
-    } else {
-      if (S == 12) launch_leaf_text<12, false>(t, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
-      else launch_leaf_text<0, false>(t, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
-    }
+    launch_leaf_text(t, direct, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
   } else {
     Launch l(t, "leaf_insert");
     const unsigned nb = (unsigned)ceil_div(n0, LVL_THREADS);
@@ -890,20 +903,21 @@ int build_impl(Tree& t, const LeafInput& in, uint64_t n0, bool direct) {
   // partition pass (LeafFinish), not by a kernel of their own
   LeafFinish leaf_finish{sc.ptr_a.ptr, sc.bitmask.ptr, sc.dids.ptr, sc.side_slots.ptr};
   const bool fuse_leaf = direct && n0 > SMALL_MAX && level_bucket_plan(t, ceil_div(n0, 2), 0).usable;
+  const TileWindow all = whole_level(n0, sc.counts.ptr);
   if (direct)
-    STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr, sc.counts.ptr, t.leaves.ptr, nullptr,
-                                           0, nullptr, nullptr, fuse_leaf));
-  else STB_TRY(finish_level<MODE_LEAF_HASH>(t, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr, sc.counts.ptr, t.leaves.ptr));
+    STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, all, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr, t.leaves.ptr,
+                                           nullptr, 0, nullptr, nullptr, fuse_leaf));
+  else
+    STB_TRY(finish_level<MODE_LEAF_HASH>(t, all, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr, t.leaves.ptr));
 
   // ---- node levels ----
   t.layers.clear();
-  int level = 0;
   uint32_t* cur = nullptr;
-  STB_TRY(run_node_levels(t, sc, sc.ptr_a.ptr, sc.ptr_b.ptr, n0, sc.counts.ptr + 1, &level, &cur, fuse_leaf ? &leaf_finish : nullptr));
+  STB_TRY(run_node_levels(t, sc, sc.ptr_a.ptr, sc.ptr_b.ptr, n0, sc.counts.ptr + 1, &cur, fuse_leaf ? &leaf_finish : nullptr));
   // `cur` now holds the single root pointer.
   t.profile_level = -1;
 
-  return finish_build(t, sc, n0, level, cur, direct);
+  return finish_build(t, sc, n0, cur);
 }
 
 // ---- streaming build from host memory --------------------------------------------------------
@@ -956,27 +970,18 @@ int stream_begin(Tree& t, Scratch& sc, StreamPlan& sp, uint64_t bound) {
   STB_CUDA(t, sc.side_slots.ensure(side_table_cap(t, bound) + 1, st));
   STB_CUDA(t, cudaMemsetAsync(sc.side_slots.ptr, 0xff, ((uint64_t)side_table_cap(t, bound) + 1) * sizeof(Slot), st));
   STB_TRY(reserve_node_workspace(t, sc, n[Lc]));  // the top of the tree, as in the one-shot build
-  {
-    bool grew = false;
-    STB_CUDA(t, sc.stream_slots.ensure(slot_off[Lc + 1], st, &grew));
-    if (grew || !sc.stream_tags_cleared) {
-      Launch l(t, "table_clear", false);
-      STB_CUDA(t, cudaMemsetAsync(sc.stream_slots.ptr, 0xff, sc.stream_slots.bytes(), st));
-      sc.stream_tags_cleared = true;
-      sc.stream_serial = 0;
-    }
-  }
+  STB_CUDA(t, sc.stream_slots.ensure(slot_off[Lc + 1], st));
+  STB_TRY(sc.stream_slots.clear_if_needed(t));
   STB_CUDA(t, cudaMemsetAsync(sc.bit_arena.ptr, 0, bit_off[Lc + 1] * 4, st));
   STB_CUDA(t, cudaMemsetAsync(sc.run_totals.ptr, 0, 2 * (Lc + 1) * 4, st));
   STB_CUDA(t, cudaMemsetAsync(sc.counts.ptr, 0, 80 * 4, st));
   STB_CUDA(t, cudaMemsetAsync(sc.dminpos.ptr, 0xff, direct_entries * 4, st));
+  STB_TRY(reset_flags(t, sc.flags.ptr));
   {
-    BuildFlags init{~0ull, 0u, 0u, 0u, 0u};
-    STB_CUDA(t, cudaMemcpyAsync(sc.flags.ptr, &init, sizeof(init), cudaMemcpyHostToDevice, st));
     std::vector<uint32_t> sizes(Lc + 2, 0);
     for (int j = 0; j <= Lc; ++j) sizes[j] = (uint32_t)n[j];
     STB_CUDA(t, cudaMemcpyAsync(sc.level_sizes.ptr, sizes.data(), sizes.size() * 4, cudaMemcpyHostToDevice, st));
-    STB_CUDA(t, cudaStreamSynchronize(st));  // `sizes` and `init` are stack memory
+    STB_CUDA(t, cudaStreamSynchronize(st));  // `sizes` is stack memory
   }
   STB_CUDA(t, t.leaves.alloc(std::min<uint64_t>(bound, direct_entries / 2 + side_table_cap(t, bound) / 2 + 2), st));
   t.layers.clear();
@@ -985,7 +990,7 @@ int stream_begin(Tree& t, Scratch& sc, StreamPlan& sp, uint64_t bound) {
     STB_CUDA(t, t.layers.back().nodes.alloc(n[j], st));
   }
   sp.serial.assign(Lc + 1, 0);
-  for (int j = 1; j <= Lc; ++j) sp.serial[j] = ++sc.stream_serial;
+  for (int j = 1; j <= Lc; ++j) sp.serial[j] = sc.stream_slots.take(1);
   return STB_OK;
 }
 
@@ -993,58 +998,37 @@ int stream_begin(Tree& t, Scratch& sc, StreamPlan& sp, uint64_t bound) {
 // chunked levels.  `n0` is the true leaf count when this is the last chunk (the ragged right edge is
 // only ever touched then), else the bound.
 int stream_chunk(Tree& t, Scratch& sc, const StreamPlan& sp, const char* body, uint64_t c, uint64_t cnt, uint64_t n0) {
-  const int S = sp.S, Lc = sp.Lc;
-  cudaStream_t st = t.stream;
+  const int Lc = sp.Lc;
   uint32_t* const ptrs = sc.ptr_arena.ptr;
   uint32_t* const bits = sc.bit_arena.ptr;
   LevelTable leaf_tab{sc.side_slots.ptr, sc.dminpos.ptr, sc.dids.ptr, side_table_cap(t, sp.bound)};
   leaf_tab.first_bits = bits;
   const uint64_t first = c * sp.C;
-  if (S == 12) launch_leaf_text<12, true>(t, body + first * S, cnt, leaf_tab, ptrs + first, sc.flags.ptr, (uint32_t)first);
-  else launch_leaf_text<0, true>(t, body + first * S, cnt, leaf_tab, ptrs + first, sc.flags.ptr, (uint32_t)first);
+  launch_leaf_text(t, true, body + first * sp.S, cnt, leaf_tab, ptrs + first, sc.flags.ptr, (uint32_t)first);
   for (int j = 0; j <= Lc; ++j) {
     const uint64_t begin = first >> j, end = ceil_div(first + cnt, 1ull << j);
     const uint64_t n_here = ceil_div(n0, 1ull << j), n_below = j ? ceil_div(n0, 1ull << (j - 1)) : 0;
-    const uint32_t fb = (uint32_t)(begin / LVL_TILE), nbk = (uint32_t)ceil_div(end - begin, LVL_TILE);
     uint32_t* lvl_ptr = ptrs + sp.ptr_off[j];
     uint32_t* lvl_bits = bits + sp.bit_off[j];
     // running total of the level: read from one copy, the new total goes to the other
-    const uint32_t* carry = sc.run_totals.ptr + (c & 1) * (Lc + 1) + j;
-    uint32_t* total = sc.run_totals.ptr + ((c + 1) & 1) * (Lc + 1) + j;
-    uint32_t* tilecnt = sc.tilecnt.ptr;
-    uint32_t* chunkcnt = tilecnt + nbk;
-    LevelTable tab = leaf_tab;
-    if (j > 0) {
-      tab = LevelTable{sc.stream_slots.ptr + sp.slot_off[j], nullptr, nullptr, table_cap(sp.n[j])};
-      tab.first_bits = lvl_bits;
+    const TileWindow w{(uint32_t)(begin / LVL_TILE), (uint32_t)ceil_div(end - begin, LVL_TILE), sc.run_totals.ptr + (c & 1) * (Lc + 1) + j,
+                       sc.run_totals.ptr + ((c + 1) & 1) * (Lc + 1) + j};
+    if (j == 0) {
+      STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, w, lvl_ptr, lvl_ptr, (uint32_t)n_here, (uint32_t)std::min<uint64_t>(n_here, first + cnt), leaf_tab,
+                                             lvl_bits, sc.tilecnt.ptr, t.leaves.ptr));
+      continue;
+    }
+    LevelTable tab{sc.stream_slots.buf.ptr + sp.slot_off[j], nullptr, nullptr, table_cap(sp.n[j])};
+    tab.first_bits = lvl_bits;
+    {
       Launch l(t, "node_insert");
       // placement by child id above the first node layer; child ids are bounded by the child level's size
       const uint32_t* child_unique = (j > 1 && t.opt.locality) ? sc.level_sizes.ptr + (j - 1) : nullptr;
-      node_insert_kernel<<<nbk, LVL_THREADS, 0, st>>>(ptrs + sp.ptr_off[j - 1], (uint32_t)n_below, (uint32_t)end, tab, lvl_ptr, child_unique,
-                                                       sp.serial[j], nullptr, nullptr, fb, nullptr);
+      node_insert_kernel<<<w.count, LVL_THREADS, 0, t.stream>>>(ptrs + sp.ptr_off[j - 1], (uint32_t)n_below, (uint32_t)end, tab, lvl_ptr, child_unique,
+                                                                sp.serial[j], nullptr, nullptr, w.first, nullptr);
     }
-    STB_CUDA(t, cudaMemsetAsync(chunkcnt, 0, (nbk / CHUNK_TILES + 1) * 4, st));
-    {
-      Launch l(t, "count_firsts");
-      count_kernel<<<(unsigned)ceil_div((uint64_t)nbk * 32, 256), 256, 0, st>>>(lvl_bits, fb, nbk, tilecnt, chunkcnt);
-    }
-    {
-      Launch l(t, "assign_ids");
-      if (j == 0)
-        assign_kernel<MODE_LEAF_DIRECT><<<nbk, LVL_THREADS, 0, st>>>(lvl_ptr, (uint32_t)n_here, tab, lvl_bits, tilecnt, chunkcnt, fb, carry, total, t.leaves.ptr, S,
-                                                                     nullptr, 0u);
-      else
-        assign_kernel<MODE_NODE><<<nbk, LVL_THREADS, 0, st>>>(lvl_ptr, (uint32_t)end, tab, lvl_bits, tilecnt, chunkcnt, fb, carry, total,
-                                                              t.layers[j - 1].nodes.ptr, S, ptrs + sp.ptr_off[j - 1], (uint32_t)n_below);
-    }
-    {
-      Launch l(t, "resolve_ids");
-      if (j == 0)
-        resolve_kernel<RESOLVE_DIRECT><<<nbk, LVL_THREADS, 0, st>>>(lvl_ptr, lvl_ptr, (uint32_t)std::min<uint64_t>(n_here, first + cnt), tab, lvl_bits, fb,
-                                                                    nullptr, nullptr);
-      else
-        resolve_kernel<RESOLVE_TABLE><<<nbk, LVL_THREADS, 0, st>>>(lvl_ptr, lvl_ptr, (uint32_t)end, tab, lvl_bits, fb, nullptr, nullptr);
-    }
+    STB_TRY(finish_level<MODE_NODE>(t, w, lvl_ptr, lvl_ptr, (uint32_t)end, (uint32_t)end, tab, lvl_bits, sc.tilecnt.ptr, t.layers[j - 1].nodes.ptr,
+                                    ptrs + sp.ptr_off[j - 1], (uint32_t)n_below));
   }
   return STB_OK;
 }
@@ -1056,18 +1040,25 @@ int stream_finish(Tree& t, Scratch& sc, const StreamPlan& sp, uint64_t n0, uint6
   const uint64_t n_top = ceil_div(n0, 1ull << Lc);
   STB_CUDA(t, cudaMemcpyAsync(sc.counts.ptr, sc.run_totals.ptr + (chunks & 1) * (Lc + 1), (Lc + 1) * 4, cudaMemcpyDeviceToDevice, st));
   STB_CUDA(t, cudaMemcpyAsync(sc.ptr_a.ptr, sc.ptr_arena.ptr + sp.ptr_off[Lc], n_top * 4, cudaMemcpyDeviceToDevice, st));
-  int more = 0;
   uint32_t* cur = nullptr;
-  STB_TRY(run_node_levels(t, sc, sc.ptr_a.ptr, sc.ptr_b.ptr, n_top, sc.counts.ptr + 1 + Lc, &more, &cur));
-  return finish_build(t, sc, n0, Lc + more, cur, true);
+  STB_TRY(run_node_levels(t, sc, sc.ptr_a.ptr, sc.ptr_b.ptr, n_top, sc.counts.ptr + 1 + Lc, &cur));
+  return finish_build(t, sc, n0, cur);
 }
 
-int ensure_copy_stream(Tree& t, Scratch& sc, uint64_t events) {
+// Queues the copy of host src[0, len) to dst in pieces of chunk_bytes, all at once on the copy
+// stream; piece i is followed by sc.chunk_events[i], which work on the compute stream waits for.
+int queue_chunk_copies(Tree& t, Scratch& sc, char* dst, const char* src, uint64_t len, uint64_t chunk_bytes) {
+  const uint64_t chunks = ceil_div(len, chunk_bytes);
   if (!sc.copy_stream) STB_CUDA(t, cudaStreamCreateWithFlags(&sc.copy_stream, cudaStreamNonBlocking));
-  while (sc.chunk_events.size() < events) {
+  while (sc.chunk_events.size() < chunks) {
     cudaEvent_t e;
     STB_CUDA(t, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     sc.chunk_events.push_back(e);
+  }
+  for (uint64_t i = 0; i < chunks; ++i) {
+    const uint64_t first = i * chunk_bytes;
+    STB_CUDA(t, cudaMemcpyAsync(dst + first, src + first, std::min(chunk_bytes, len - first), cudaMemcpyHostToDevice, sc.copy_stream));
+    STB_CUDA(t, cudaEventRecord(sc.chunk_events[i], sc.copy_stream));
   }
   return STB_OK;
 }
@@ -1081,7 +1072,7 @@ bool streaming_applies(const Tree& t, uint64_t n0_bound) {
 int build_streaming(Tree& t, const char* h_body, uint64_t body_len) {
   const int S = t.S;
   const uint64_t n0 = body_len / (uint64_t)S;
-  if (!streaming_applies(t, n0)) return -1;
+  if (!streaming_applies(t, n0)) return NOT_APPLICABLE;
   cudaStream_t st = t.stream;
   t.clear();
   Scratch& sc = workspace_of(t);
@@ -1089,14 +1080,8 @@ int build_streaming(Tree& t, const char* h_body, uint64_t body_len) {
   STB_CUDA(t, t.staging.ensure(n0 * (uint64_t)S + 16, st));
   STB_TRY(stream_begin(t, sc, sp, n0));
   const uint64_t C = sp.C, chunks = ceil_div(n0, C);
-  // all chunk copies are queued at once on their own stream; compute waits chunk by chunk
-  STB_TRY(ensure_copy_stream(t, sc, chunks));
   char* text = t.staging.ptr;
-  for (uint64_t c = 0; c < chunks; ++c) {
-    const uint64_t first = c * C, cnt = std::min<uint64_t>(C, n0 - first);
-    STB_CUDA(t, cudaMemcpyAsync(text + first * S, h_body + first * S, cnt * S, cudaMemcpyHostToDevice, sc.copy_stream));
-    STB_CUDA(t, cudaEventRecord(sc.chunk_events[c], sc.copy_stream));
-  }
+  STB_TRY(queue_chunk_copies(t, sc, text, h_body, n0 * S, C * S));
   for (uint64_t c = 0; c < chunks; ++c) {
     STB_CUDA(t, cudaStreamWaitEvent(st, sc.chunk_events[c], 0));
     STB_TRY(stream_chunk(t, sc, sp, text, c, std::min<uint64_t>(C, n0 - c * C), n0));
@@ -1112,7 +1097,7 @@ int build_streaming(Tree& t, const char* h_body, uint64_t body_len) {
 int build_streaming_fasta(Tree& t, const char* h_text, uint64_t len) {
   const int S = t.S;
   const uint64_t bound = len / (uint64_t)S;
-  if (!streaming_applies(t, bound)) return -1;
+  if (!streaming_applies(t, bound)) return NOT_APPLICABLE;
   cudaStream_t st = t.stream;
   t.clear();
   Scratch& sc = workspace_of(t);
@@ -1123,15 +1108,10 @@ int build_streaming_fasta(Tree& t, const char* h_text, uint64_t len) {
   const uint64_t C = sp.C;
   const uint64_t text_chunk = std::max<uint64_t>(FASTA_STREAM_ALIGN, (C * S / 2) & ~(FASTA_STREAM_ALIGN - 1));
   const uint64_t text_chunks = ceil_div(len, text_chunk);
-  STB_TRY(ensure_copy_stream(t, sc, text_chunks));
   STB_TRY(fasta_stream_begin(t, sc.fasta, text_chunk));
   char* text = t.staging.ptr;
   char* body = sc.stream_body.ptr;
-  for (uint64_t i = 0; i < text_chunks; ++i) {
-    const uint64_t first = i * text_chunk, cnt = std::min<uint64_t>(text_chunk, len - first);
-    STB_CUDA(t, cudaMemcpyAsync(text + first, h_text + first, cnt, cudaMemcpyHostToDevice, sc.copy_stream));
-    STB_CUDA(t, cudaEventRecord(sc.chunk_events[i], sc.copy_stream));
-  }
+  STB_TRY(queue_chunk_copies(t, sc, text, h_text, len, text_chunk));
   uint64_t built = 0;  // leaf chunks already built
   uint64_t body_len = 0;
   for (uint64_t i = 0; i < text_chunks; ++i) {
@@ -1165,7 +1145,7 @@ int build_dispatch(Tree& t, const LeafInput& in, uint64_t n0) {
   const bool try_direct = t.S <= 12;
   if (try_direct) {
     const int s = build_impl(t, in, n0, true);
-    if (s != -1) return s;
+    if (s != NOT_APPLICABLE) return s;
   }
   if (n0 > 268000000ull)
     return t.fail(STB_ERR_TOO_LARGE, "hash-table leaf level supports at most 268M leaf positions in this version");
@@ -1191,17 +1171,9 @@ int build_upper_levels(Tree& t, const uint32_t* d_ptrs, uint64_t n, bool at_leas
   Scratch& sc = workspace_of(t);
   STB_TRY(reserve_node_workspace(t, sc, n));
   STB_CUDA(t, cudaMemcpyAsync(sc.ptr_a.ptr, d_ptrs, n * 4, cudaMemcpyDeviceToDevice, st));
-  int level = 0;
   uint32_t* cur = nullptr;
-  STB_TRY(run_node_levels(t, sc, sc.ptr_a.ptr, sc.ptr_b.ptr, n, sc.counts.ptr, &level, &cur));
-  std::vector<uint32_t> counts(level);
-  uint32_t root = PTR_NULL;
-  STB_CUDA(t, cudaMemcpyAsync(counts.data(), sc.counts.ptr, counts.size() * 4, cudaMemcpyDeviceToHost, st));
-  STB_CUDA(t, cudaMemcpyAsync(&root, cur, 4, cudaMemcpyDeviceToHost, st));
-  STB_CUDA(t, cudaStreamSynchronize(st));
-  STB_CUDA(t, cudaGetLastError());
-  for (int k = 0; k < level; ++k) t.layers[k].count = counts[k];
-  t.root = root;
+  STB_TRY(run_node_levels(t, sc, sc.ptr_a.ptr, sc.ptr_b.ptr, n, sc.counts.ptr, &cur));
+  STB_TRY(read_back(t, sc.counts.ptr, false, cur));
   t.built = true;
   return STB_OK;
 }
@@ -1214,16 +1186,13 @@ int dist_leaf_direct_minpos(Ctx& ctx, const char* d_body, uint64_t n_local, uint
   if (n_local == 0) return STB_OK;
   DevBuf<BuildFlags> flags;
   STB_CUDA(ctx, flags.alloc(1, ctx.stream));
-  BuildFlags init{~0ull, 0u, 0u, 0u, 0u};
-  STB_CUDA(ctx, cudaMemcpyAsync(flags.ptr, &init, sizeof(init), cudaMemcpyHostToDevice, ctx.stream));
-  LevelTable tab{nullptr, dminpos, nullptr, 0u};
-  if (ctx.S == 12) launch_leaf_text<12, true>(ctx, d_body, n_local, tab, tmp, flags.ptr, (uint32_t)gpos0);
-  else launch_leaf_text<0, true>(ctx, d_body, n_local, tab, tmp, flags.ptr, (uint32_t)gpos0);
+  STB_TRY(reset_flags(ctx, flags.ptr));
+  launch_leaf_text(ctx, true, d_body, n_local, LevelTable{nullptr, dminpos, nullptr, 0u}, tmp, flags.ptr, (uint32_t)gpos0);
   BuildFlags h{};
   STB_CUDA(ctx, cudaMemcpyAsync(&h, flags.ptr, sizeof(h), cudaMemcpyDeviceToHost, ctx.stream));
   STB_CUDA(ctx, cudaStreamSynchronize(ctx.stream));
   STB_CUDA(ctx, cudaGetLastError());
-  if (h.bad_symbol != ~0ull) return ctx.fail(STB_ERR_UNKNOWN_SYMBOL, unknown_symbol_message((int)(h.bad_symbol & 0xff)));
+  STB_TRY(check_flags(ctx, h));
   *non_acgt = (int)h.non_acgt;
   return STB_OK;
 }
@@ -1234,8 +1203,8 @@ int build_from_body(Tree& t, const char* d_body, uint64_t body_len) {
   return build_dispatch(t, in, body_len / (uint64_t)t.S);
 }
 
-// Host text: overlap the copy with the build when the input is large enough; -1 = not applicable
-// (small input, dna_size > 12, or non-ACGT symbols), the caller copies and builds in one shot.
+// Host text: overlap the copy with the build when the input is large enough; NOT_APPLICABLE (small
+// input, dna_size > 12, or non-ACGT symbols): the caller copies and builds in one shot.
 int build_from_host_body(Tree& t, const char* h_body, uint64_t body_len) { return build_streaming(t, h_body, body_len); }
 int build_from_host_fasta(Tree& t, const char* h_text, uint64_t len) { return build_streaming_fasta(t, h_text, len); }
 

@@ -265,7 +265,7 @@ int stb_build_from_body(stb_tree* tree, const char* body, uint64_t len, int memo
   STB_TRY(use_device(tree));
   if (memory == STB_HOST) {  // large host inputs: build chunk by chunk behind the copy
     const int s = build_from_host_body(*tree, body, len);
-    if (s != -1) return s;
+    if (s != NOT_APPLICABLE) return s;
   }
   DevBuf<char> hold;
   const char* d = nullptr;
@@ -280,7 +280,7 @@ int stb_build_from_fasta(stb_tree* tree, const char* text, uint64_t len, int mem
   if (len == 0) return t.fail(STB_ERR_EMPTY, "input holds fewer than dna_size bases");
   if (memory == STB_HOST) {  // large host inputs: extract and build chunk by chunk behind the copy
     const int s = build_from_host_fasta(t, text, len);
-    if (s != -1) return s;
+    if (s != NOT_APPLICABLE) return s;
   }
   DevBuf<char> hold;
   const char* d = nullptr;

@@ -103,8 +103,10 @@ int pack_body(Ctx& ctx, const char* d_body, uint64_t n_leaves, unsigned long lon
 // build.cu -------------------------------------------------------------------------
 int build_from_body(Tree& t, const char* d_body, uint64_t body_len);
 int build_from_leaves(Tree& t, const unsigned long long* d_leaves, uint64_t n);
-int build_from_host_body(Tree& t, const char* h_body, uint64_t body_len);  // streaming; -1 = use the one-shot path
-int build_from_host_fasta(Tree& t, const char* h_text, uint64_t len);      // streaming incl. body extraction; -1 = use the one-shot path
+// status of a path that does not apply to this input (the caller takes another one); every stb_status is >= 0
+constexpr int NOT_APPLICABLE = -1;
+int build_from_host_body(Tree& t, const char* h_body, uint64_t body_len);  // streaming, or NOT_APPLICABLE: use the one-shot path
+int build_from_host_fasta(Tree& t, const char* h_text, uint64_t len);      // streaming incl. body extraction, or NOT_APPLICABLE
 int build_upper_levels(Tree& t, const uint32_t* d_ptrs, uint64_t n, bool at_least_one);
 int dist_leaf_direct_minpos(Ctx& ctx, const char* d_body, uint64_t n_local, uint64_t gpos0, uint32_t* dminpos, uint32_t* tmp,
                             int* non_acgt);
