@@ -129,11 +129,16 @@ partition_tile(const uint32_t bx, const uint32_t by, const uint32_t* __restrict_
           l = __ldcg(leaf.words + 2 * (uint64_t)i);
         }
         // (no bitmap: every word is still a code, as the sharded build's replicated leaf table leaves them)
-        const uint32_t firsts = leaf.first_bits ? __ldg(leaf.first_bits + (i >> 4)) >> ((2u * i) & 31u) : 0u;
-        if (!(firsts & 1u)) l = finish_leaf(l, leaf);
-        if (pair && !(firsts & 2u)) r = finish_leaf(r, leaf);
-        if (pair) reinterpret_cast<uint2*>(leaf.words)[i] = make_uint2(l, r);
-        else leaf.words[2 * (uint64_t)i] = l;
+        uint32_t finished = leaf.first_bits ? __ldg(leaf.first_bits + (i >> 4)) : 0u;
+        if (leaf.done_bits) finished |= __ldg(leaf.done_bits + (i >> 4));
+        finished = (finished >> ((2u * i) & 31u)) | (pair ? 0u : 2u);
+        if (!(finished & 1u)) l = finish_leaf(l, leaf);
+        if (!(finished & 2u)) r = finish_leaf(r, leaf);
+        // only a pair with a word finished here goes back to memory
+        if ((finished & 3u) != 3u) {
+          if (pair) reinterpret_cast<uint2*>(leaf.words)[i] = make_uint2(l, r);
+          else leaf.words[2 * (uint64_t)i] = l;
+        }
         schild[o] = make_uint2(l, r);
       }
     }

@@ -64,6 +64,7 @@ struct LeafFinish {
   const uint32_t* first_bits = nullptr;  // the leaf level's first occurrences
   const uint32_t* dids = nullptr;        // id by canonical 2-bit code
   const Slot* side = nullptr;            // leaves outside ACGT: min-position per leaf (its word holds the id)
+  const uint32_t* done_bits = nullptr;   // later occurrences the leaf kernel already finished (null: none)
 };
 
 struct BucketWorkspace {

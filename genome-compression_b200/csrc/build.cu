@@ -158,50 +158,74 @@ __device__ __forceinline__ uint32_t reverse_2bit_24(uint32_t c) {
   return ((r & 0x555555u) << 1) | ((r >> 1) & 0x555555u);
 }
 
+// LOOKUP (one-shot build, the leaves after a prefix whose ids are already assigned): a leaf whose code
+// has an id in tab.dids is a later occurrence of a prefix leaf; it gets its finished pointer here and
+// its bit in done_bits (indexed by position; a warp covers one word), and skips the min-position
+// table.  Every other leaf takes the insert below and stays pending.
+template <bool LOOKUP>
+__device__ __forceinline__ bool acgt12_leaf(const uint8_t* smem, const uint8_t* tile, uint32_t j, uint64_t tile_first, const LevelTable& tab,
+                                            uint32_t* __restrict__ tmp, BuildFlags* flags, uint32_t pos0) {
+  const uint32_t* words = reinterpret_cast<const uint32_t*>(tile);
+  uint32_t c0, c1, c2;
+  const bool ok = acgt_word_to_2bit(words[3 * j], c0) & acgt_word_to_2bit(words[3 * j + 1], c1) & acgt_word_to_2bit(words[3 * j + 2], c2);
+  if (!ok) {  // a symbol outside ACGT: the general 4-bit pack of this one leaf, into the side table
+    uint32_t bad = 0xFFFFFFFFu, f4;
+    const unsigned long long v = pack_leaf<12>(smem, tile, j, 12, bad);
+    if (bad != 0xFFFFFFFFu) {
+      uint32_t ch = tile[bad];
+      if (ch >= 'a' && ch <= 'z') ch -= 32;
+      // (a lookup launch starts at leaf pos0 of the body its caller holds: offsets count from the body's start)
+      const uint64_t text0 = LOOKUP ? (uint64_t)pos0 * 12 : 0;
+      atomicMin(&flags->bad_symbol, ((text0 + tile_first * 12 + bad) << 8) | ch);
+    }
+    const unsigned long long canon = canonical_leaf(v, 12, f4);
+    const uint32_t side = side_insert(tab, canon, pos0 + (uint32_t)(tile_first + j), flags);
+    tmp[tile_first + j] = side == 0xffffffffu ? 0u : (LEAF_SIDE | side | f4);
+    return false;
+  }
+  const uint32_t c = c0 | (c1 << 8) | (c2 << 16);
+  const uint32_t t = ~c & 0xFFFFFFu, m = reverse_2bit_24(c), i = ~m & 0xFFFFFFu;
+  uint32_t best = c, f = 0;
+  if (t < best) { best = t; f = TRANSPOSE; }
+  if (m < best) { best = m; f = MIRROR; }
+  if (i < best) { best = i; f = MIRROR | TRANSPOSE; }
+  if (c == m) f |= INVARIANT;
+  if (LOOKUP) {
+    const uint32_t id = __ldcg(tab.dids + best);
+    if (id != 0xffffffffu) {
+      tmp[tile_first + j] = finish_pointer(id, f);
+      return true;
+    }
+  }
+  const uint32_t pos = pos0 + (uint32_t)(tile_first + j);
+  if (__ldcg(tab.dminpos + best) > pos) {
+    const uint32_t old = atomicMin(tab.dminpos + best, pos);
+    if (tab.first_bits && old > pos) {
+      toggle_bit(tab.first_bits, pos);
+      if (old != 0xffffffffu) toggle_bit(tab.first_bits, old);
+    }
+  }
+  tmp[tile_first + j] = best | f;
+  return false;
+}
+
+template <bool LOOKUP>
 __global__ void __launch_bounds__(PACK_THREADS)
 leaf_insert_acgt12_kernel(const char* __restrict__ body, uint64_t n_leaves, LevelTable tab, uint32_t* __restrict__ tmp,
-                          BuildFlags* flags, uint32_t pos0) {
+                          BuildFlags* flags, uint32_t pos0, uint32_t* __restrict__ done_bits) {
   extern __shared__ __align__(16) uint8_t smem[];
   uint8_t* tile = smem + 256;  // same layout as the general kernel (the table area is unused here)
   const uint64_t tile_first = (uint64_t)blockIdx.x * PACK_TILE_LEAVES;
   const uint32_t here = (uint32_t)min((uint64_t)PACK_TILE_LEAVES, n_leaves - tile_first);
   stage_text_tile(smem, tile, body + tile_first * 12, here * 12u);
-  const uint32_t* words = reinterpret_cast<const uint32_t*>(tile);
 #pragma unroll
   for (int it = 0; it < PACK_LEAVES_PER_THREAD; ++it) {
     const uint32_t j = it * PACK_THREADS + threadIdx.x;
-    if (j >= here) continue;
-    uint32_t c0, c1, c2;
-    const bool ok = acgt_word_to_2bit(words[3 * j], c0) & acgt_word_to_2bit(words[3 * j + 1], c1) & acgt_word_to_2bit(words[3 * j + 2], c2);
-    if (!ok) {  // a symbol outside ACGT: the general 4-bit pack of this one leaf, into the side table
-      uint32_t bad = 0xFFFFFFFFu, f4;
-      const unsigned long long v = pack_leaf<12>(smem, tile, j, 12, bad);
-      if (bad != 0xFFFFFFFFu) {
-        uint32_t ch = tile[bad];
-        if (ch >= 'a' && ch <= 'z') ch -= 32;
-        atomicMin(&flags->bad_symbol, ((tile_first * 12 + bad) << 8) | ch);
-      }
-      const unsigned long long canon = canonical_leaf(v, 12, f4);
-      const uint32_t side = side_insert(tab, canon, pos0 + (uint32_t)(tile_first + j), flags);
-      tmp[tile_first + j] = side == 0xffffffffu ? 0u : (LEAF_SIDE | side | f4);
-      continue;
+    const bool done = j < here && acgt12_leaf<LOOKUP>(smem, tile, j, tile_first, tab, tmp, flags, pos0);
+    if (LOOKUP) {  // pos0 is a multiple of 32: the warp's 32 positions are one word, lane 0 stores it whole
+      const uint32_t word = __ballot_sync(0xffffffffu, done);
+      if ((threadIdx.x & 31) == 0 && j < here) done_bits[(pos0 + (uint32_t)(tile_first + j)) >> 5] = word;
     }
-    const uint32_t c = c0 | (c1 << 8) | (c2 << 16);
-    const uint32_t t = ~c & 0xFFFFFFu, m = reverse_2bit_24(c), i = ~m & 0xFFFFFFu;
-    uint32_t best = c, f = 0;
-    if (t < best) { best = t; f = TRANSPOSE; }
-    if (m < best) { best = m; f = MIRROR; }
-    if (i < best) { best = i; f = MIRROR | TRANSPOSE; }
-    if (c == m) f |= INVARIANT;
-    const uint32_t pos = pos0 + (uint32_t)(tile_first + j);
-    if (__ldcg(tab.dminpos + best) > pos) {
-      const uint32_t old = atomicMin(tab.dminpos + best, pos);
-      if (tab.first_bits && old > pos) {
-        toggle_bit(tab.first_bits, pos);
-        if (old != 0xffffffffu) toggle_bit(tab.first_bits, old);
-      }
-    }
-    tmp[tile_first + j] = best | f;
   }
 }
 
@@ -556,6 +580,7 @@ struct Scratch {
   DevBuf<uint32_t> ptr_a, ptr_b, aux, bitmask, counts, dminpos, dids;
   DevBuf<uint32_t> lvl_bits[2], lvl_multi[2];  // node levels: first occurrences / first occurrences that occur again, by level parity
   DevBuf<uint32_t> tilecnt;                    // first occurrences per tile, then per chunk of tiles (count_kernel)
+  DevBuf<uint32_t> leaf_done, leaf_carry;      // leaf level after a prefix: positions finished by the leaf kernel; first occurrences in the prefix
   DevBuf<Slot> side_slots;
   DevBuf<BuildFlags> flags;
   DevBuf<uint32_t> root;
@@ -593,12 +618,16 @@ uint32_t side_table_cap(const Tree& t, uint64_t n0) {
 uint32_t table_cap(uint64_t n) { return (uint32_t)std::min<uint64_t>(std::max<uint64_t>(1024, 2 * n), 0x1ffffffeull); }
 uint64_t bitmap_words(uint64_t n) { return ceil_div(n, LVL_TILE) * (LVL_TILE / 32); }
 
-// The leaf level from ASCII text.  ACGT leaves of length 12 next to the direct table take the SWAR kernel.
-void launch_leaf_text(Ctx& ctx, bool direct, const char* body, uint64_t n, LevelTable tab, uint32_t* tmp, BuildFlags* flags, uint32_t pos0 = 0) {
+// The leaf level from ASCII text.  ACGT leaves of length 12 next to the direct table take the SWAR kernel;
+// with `done_bits` (a multiple of 32 in pos0) that kernel's lookup mode.
+void launch_leaf_text(Ctx& ctx, bool direct, const char* body, uint64_t n, LevelTable tab, uint32_t* tmp, BuildFlags* flags, uint32_t pos0 = 0,
+                      uint32_t* done_bits = nullptr) {
   const unsigned grid = (unsigned)ceil_div(n, PACK_TILE_LEAVES);
   const size_t smem = pack_smem_bytes(ctx.S);
   Launch l(ctx, "leaf_insert");
-  if (ctx.S == 12 && direct) leaf_insert_acgt12_kernel<<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, tab, tmp, flags, pos0);
+  if (ctx.S == 12 && direct && done_bits)
+    leaf_insert_acgt12_kernel<true><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, tab, tmp, flags, pos0, done_bits);
+  else if (ctx.S == 12 && direct) leaf_insert_acgt12_kernel<false><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, tab, tmp, flags, pos0, nullptr);
   else if (ctx.S == 12) leaf_insert_text_kernel<12, false><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, ctx.S, tab, tmp, flags, pos0);
   else if (direct) leaf_insert_text_kernel<0, true><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, ctx.S, tab, tmp, flags, pos0);
   else leaf_insert_text_kernel<0, false><<<grid, PACK_THREADS, smem, ctx.stream>>>(body, n, ctx.S, tab, tmp, flags, pos0);
@@ -891,24 +920,50 @@ int build_impl(Tree& t, const LeafInput& in, uint64_t n0, bool direct) {
   const uint64_t leaf_store = direct ? std::min<uint64_t>(n0, direct_entries / 2 + side_table_cap(t, n0) / 2 + 2) : n0;
   STB_CUDA(t, t.leaves.alloc(leaf_store, st));
 
-  if (in.body) {
-    launch_leaf_text(t, direct, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
-  } else {
-    Launch l(t, "leaf_insert");
-    const unsigned nb = (unsigned)ceil_div(n0, LVL_THREADS);
-    if (direct) leaf_insert_u64_kernel<true><<<nb, LVL_THREADS, 0, st>>>(in.leaves, (uint32_t)n0, S, tab, sc.ptr_a.ptr, sc.flags.ptr);
-    else leaf_insert_u64_kernel<false><<<nb, LVL_THREADS, 0, st>>>(in.leaves, (uint32_t)n0, S, tab, sc.ptr_a.ptr, sc.flags.ptr);
-  }
   // direct leaf level under a bucketed first node level: the later occurrences are resolved by that level's
   // partition pass (LeafFinish), not by a kernel of their own
   LeafFinish leaf_finish{sc.ptr_a.ptr, sc.bitmask.ptr, sc.dids.ptr, sc.side_slots.ptr};
   const bool fuse_leaf = direct && n0 > SMALL_MAX && level_bucket_plan(t, ceil_div(n0, 2), 0).usable;
-  const TileWindow all = whole_level(n0, sc.counts.ptr);
-  if (direct)
-    STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, all, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr, t.leaves.ptr,
-                                           nullptr, 0, nullptr, nullptr, fuse_leaf));
-  else
-    STB_TRY(finish_level<MODE_LEAF_HASH>(t, all, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr, t.leaves.ptr));
+  // ACGT text at S = 12 in two windows: the first P leaves as below, then the rest, which look up the ids the
+  // prefix assigned (as in the streaming build, they are final) and finish most of their own pointers; the
+  // partition pass then only finishes codes that had not occurred in the prefix.  P is whole tiles of both the
+  // leaf kernel and the level kernels.
+  const uint64_t prefix_log2 = std::min<uint64_t>(t.opt.leaf_prefix_log2, 40);
+  const uint64_t P = 1ull << std::max<uint64_t>(prefix_log2, 10);
+  const bool split = in.body && direct && S == 12 && fuse_leaf && prefix_log2 > 0 && n0 >= 2 * P;
+  static_assert(1024 % LVL_TILE == 0 && 1024 % PACK_TILE_LEAVES == 0, "the smallest prefix is whole tiles");
+  if (split) {
+    STB_CUDA(t, sc.leaf_done.ensure(bitmap_words(n0), st));
+    STB_CUDA(t, sc.leaf_carry.ensure(1, st));
+    // an id that is not ~0 is final (assign_tile writes it); the suffix kernel writes every done word from P on
+    STB_CUDA(t, cudaMemsetAsync(sc.dids.ptr, 0xff, direct_entries * 4, st));
+    STB_CUDA(t, cudaMemsetAsync(sc.leaf_done.ptr, 0, P / 8, st));
+    leaf_finish.done_bits = sc.leaf_done.ptr;
+    launch_leaf_text(t, direct, in.body, P, tab, sc.ptr_a.ptr, sc.flags.ptr);
+    const TileWindow prefix{0u, (uint32_t)(P / LVL_TILE), nullptr, sc.leaf_carry.ptr};
+    STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, prefix, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr,
+                                           t.leaves.ptr, nullptr, 0, nullptr, nullptr, true));
+    launch_leaf_text(t, direct, in.body + P * 12, n0 - P, tab, sc.ptr_a.ptr + P, sc.flags.ptr, (uint32_t)P, sc.leaf_done.ptr);
+    const TileWindow suffix{(uint32_t)(P / LVL_TILE), (uint32_t)ceil_div(n0 - P, LVL_TILE), sc.leaf_carry.ptr, sc.counts.ptr};
+    STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, suffix, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr,
+                                           t.leaves.ptr, nullptr, 0, nullptr, nullptr, true));
+  } else {
+    if (in.body) {
+      launch_leaf_text(t, direct, in.body, n0, tab, sc.ptr_a.ptr, sc.flags.ptr);
+    } else {
+      Launch l(t, "leaf_insert");
+      const unsigned nb = (unsigned)ceil_div(n0, LVL_THREADS);
+      if (direct) leaf_insert_u64_kernel<true><<<nb, LVL_THREADS, 0, st>>>(in.leaves, (uint32_t)n0, S, tab, sc.ptr_a.ptr, sc.flags.ptr);
+      else leaf_insert_u64_kernel<false><<<nb, LVL_THREADS, 0, st>>>(in.leaves, (uint32_t)n0, S, tab, sc.ptr_a.ptr, sc.flags.ptr);
+    }
+    const TileWindow all = whole_level(n0, sc.counts.ptr);
+    if (direct)
+      STB_TRY(finish_level<MODE_LEAF_DIRECT>(t, all, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr,
+                                             t.leaves.ptr, nullptr, 0, nullptr, nullptr, fuse_leaf));
+    else
+      STB_TRY(finish_level<MODE_LEAF_HASH>(t, all, sc.ptr_a.ptr, sc.ptr_a.ptr, (uint32_t)n0, (uint32_t)n0, tab, sc.bitmask.ptr, sc.tilecnt.ptr,
+                                           t.leaves.ptr));
+  }
 
   // ---- node levels ----
   t.layers.clear();

@@ -33,6 +33,8 @@ struct Options {
   uint64_t reserve_pipeline = 1;         // a build also reserves the scratch of sort_tree and decode (the compress path always sorts)
   uint64_t stream_chunk_log2 = 24;       // leaves per chunk of the streaming host build
   uint64_t stream_min_chunks = 4;        // smaller host inputs are copied and built in one shot
+  uint64_t leaf_prefix_log2 = 25;        // one-shot ACGT-12 leaf level: after this many positions the ids seen so far are final and
+                                         // the rest of the leaves look them up (build.cu: leaf_insert_acgt12_kernel); 0 = one window
   uint64_t profile_levels = 0;           // the kernel timings of stb_profile_read are kept per level ("name@L3")
 };
 

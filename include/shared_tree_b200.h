@@ -66,7 +66,7 @@ int stb_release_workspace(stb_tree* tree);
 /* Tunables of the build (thresholds between its code paths; DESIGN.md §4).  Defaults are the
  * measured optimum; tests lower them to push small inputs through the large-input paths.
  * Names: "bucket_min", "bucket_levels", "bucket_cap", "partition_threads", "dedup_threads", "bucket_slack_permille", "bucket_headroom", "child_filter", "locality",
- * "coop_max", "reserve_pipeline", "side_table_slots", "stream_chunk_log2", "stream_min_chunks", "profile_levels".  Unknown name: STB_ERR_INVALID_ARG. */
+ * "coop_max", "reserve_pipeline", "side_table_slots", "stream_chunk_log2", "stream_min_chunks", "leaf_prefix_log2", "profile_levels".  Unknown name: STB_ERR_INVALID_ARG. */
 int stb_set_option(stb_tree* tree, const char* name, uint64_t value);
 int stb_get_option(const stb_tree* tree, const char* name, uint64_t* value);
 
