@@ -38,9 +38,11 @@ constexpr int DD_CAP = 3072;                    // records of a final bucket, he
 constexpr int DD_SLOTS = 4096;                  // shared-memory table: key 8 B + min-position 4 B per slot
 constexpr size_t DD_SMEM = (size_t)DD_SLOTS * 12 + DD_SLOTS / 8;
 
-// overflow[0]: the level cannot be deduplicated on chip (a first-pass bucket outgrew its region, or a final
-// bucket holds more distinct keys than the shared-memory table) - build.cu re-runs it through the table in
-// HBM.  overflow[1]: a final bucket outgrew its fixed region - the exact-size pass takes over.
+// overflow[0]: the level cannot be deduplicated on chip - build.cu re-runs it through the table in HBM.  It is 1
+// when a first-pass bucket outgrew its region and 2 when a final bucket holds more distinct keys than the
+// shared-memory table.  overflow[1]: a final bucket outgrew its fixed region - the exact-size pass takes over; it
+// becomes 2 once bucket_dedup_chunked_kernel has taken a bucket.  Every reader only tests for non-zero; the values
+// tell the outcomes apart for the profile (build.cu: dedup_outcome).
 __device__ __forceinline__ bool exact_pass_wanted(const uint32_t* overflow) { return overflow[1] != 0u && overflow[0] == 0u; }
 
 __device__ __forceinline__ unsigned long long bucket_hash(unsigned long long key) {
@@ -505,6 +507,7 @@ bucket_dedup_chunked_kernel(const unsigned long long* __restrict__ keys, const u
   for (uint32_t b = blockIdx.x; b < nb; b += gridDim.x) {
     const uint32_t base = __ldg(off + b), count = __ldg(off + b + 1) - base;
     if (count <= (uint32_t)DD_CAP) continue;  // done by bucket_dedup_kernel<.., EXACT>
+    if (tid == 0) overflow[1] = 2u;
     for (uint32_t i = tid; i < DD_SLOTS; i += DD_THREADS) {
       tkey[i] = EMPTY_KEY;
       tmin[i] = 0xffffffffu;
@@ -532,7 +535,7 @@ bucket_dedup_chunked_kernel(const unsigned long long* __restrict__ keys, const u
     }
     __syncthreads();
     if (full) {
-      if (tid == 0) overflow[0] = 1u;
+      if (tid == 0) overflow[0] = 2u;
       return;  // the whole level is done again through the table in HBM
     }
     for (uint32_t i = tid; i < count; i += DD_THREADS) {

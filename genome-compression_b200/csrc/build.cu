@@ -585,6 +585,9 @@ struct Scratch {
   DevBuf<BuildFlags> flags;
   DevBuf<uint32_t> root;
   BucketWorkspace bucket;
+  // profiling on: the two overflow words of every on-chip level of the current build, and each level's profile tag
+  DevBuf<uint32_t> outcomes;
+  std::vector<int> outcome_levels;
   // The node levels' table (the hashed leaf level uses it untagged), and the streaming build's
   // per-level tables.  They count their own epochs: a reset of one counter must never make a tag
   // that is still stored in the other table current again.
@@ -708,6 +711,17 @@ int reserve_node_workspace(Tree& t, Scratch& sc, uint64_t n_cur) {
   return STB_OK;
 }
 
+// On-chip levels whose outcome one build can report (a build has fewer than 32 node levels).
+constexpr size_t MAX_OUTCOMES = 64;
+
+// The profile class of an on-chip level's outcome, from its two overflow words (bucket.cu: exact_pass_wanted).
+const char* dedup_outcome(uint32_t first, uint32_t exact) {
+  if (first == 1u) return "dedup_fallback_first_pass";
+  if (first != 0u) return "dedup_fallback_distinct";
+  if (exact == 2u) return "dedup_chunked";
+  return exact ? "dedup_exact" : "dedup_on_chip";
+}
+
 // The on-chip (bucketed) plan of node level `level` with n_next positions, or an unusable one.
 BucketPlan level_bucket_plan(const Tree& t, uint64_t n_next, int level) {
   return (n_next >= t.opt.bucket_min && (uint64_t)level < t.opt.bucket_levels) ? bucket_plan(n_next, t.opt) : BucketPlan{};
@@ -723,6 +737,7 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
   cudaStream_t st = t.stream;
   int level = 0;
   STB_TRY(sc.slots.clear_if_needed(t));  // never cleared between levels (EpochTable)
+  sc.outcome_levels.clear();
   const int level_tag0 = t.profile_level;  // the caller's level of `cur` (leaf pointers: 0), or -1
   do {
     if (level_tag0 >= 0) t.profile_level = level_tag0 + level + 1;
@@ -802,6 +817,11 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
       // on chip (bucket.cu); the hash-table kernels below then run only if a bucket overflowed
       STB_TRY(bucket_dedup_level(t, sc.bucket, pl, cur, (uint32_t)n_cur, (uint32_t)n_next, child_first, child_multi, sc.aux.ptr, first_bits, multi_bits,
                                  &overflow, level == 0 ? leaf : nullptr));
+      if (t.profiling && sc.outcome_levels.size() < MAX_OUTCOMES) {  // read_back reports the outcome (dedup_outcome)
+        STB_CUDA(t, sc.outcomes.ensure(2 * MAX_OUTCOMES, st));
+        STB_CUDA(t, cudaMemcpyAsync(sc.outcomes.ptr + 2 * sc.outcome_levels.size(), overflow, 8, cudaMemcpyDeviceToDevice, st));
+        sc.outcome_levels.push_back(t.profile_level);
+      }
       Launch l(t, "bucket_fallback");
       bitmaps_reset_kernel<<<296, 256, 0, st>>>(first_bits, multi_bits, (uint32_t)bitmap_words(n_next), overflow);
     }
@@ -826,21 +846,28 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
 // Copies the item counts at counts_dev (the leaves' first when `leaves`, then one per layer of
 // t.layers) and the root pointer at root_dev to the host, with the build flags when `flags_dev` is
 // given, and waits.  The flags are reported first, then a count at the index ceiling; the tree is
-// cleared when either fails.  Otherwise fills in the counts and the root.
+// cleared when either fails.  Otherwise fills in the counts and the root, and adds the outcome of every
+// on-chip level that run_node_levels recorded (profiling on) to the profile.
 int read_back(Tree& t, const uint32_t* counts_dev, bool leaves, const uint32_t* root_dev, const BuildFlags* flags_dev = nullptr) {
   cudaStream_t st = t.stream;
+  Scratch& sc = workspace_of(t);
   const size_t first_layer = leaves ? 1 : 0;  // index of t.layers[0]'s count
   std::vector<uint32_t> counts(first_layer + t.layers.size());
+  std::vector<uint32_t> outcomes(2 * sc.outcome_levels.size());
   BuildFlags flags = NO_FLAGS;
   uint32_t root = PTR_NULL;
   STB_CUDA(t, cudaMemcpyAsync(counts.data(), counts_dev, counts.size() * 4, cudaMemcpyDeviceToHost, st));
   if (flags_dev) STB_CUDA(t, cudaMemcpyAsync(&flags, flags_dev, sizeof(flags), cudaMemcpyDeviceToHost, st));
   STB_CUDA(t, cudaMemcpyAsync(&root, root_dev, 4, cudaMemcpyDeviceToHost, st));
+  if (!outcomes.empty()) STB_CUDA(t, cudaMemcpyAsync(outcomes.data(), sc.outcomes.ptr, outcomes.size() * 4, cudaMemcpyDeviceToHost, st));
   STB_CUDA(t, cudaStreamSynchronize(st));
   STB_CUDA(t, cudaGetLastError());
 
   int s = check_flags(t, flags);
   if (s == STB_OK && flags.non_acgt) s = NOT_APPLICABLE;  // only the direct leaf level raises it: the input needs the hash-table one
+  if (s == STB_OK)  // not for an attempt that another path repeats
+    for (size_t k = 0; k < sc.outcome_levels.size(); ++k) t.account(dedup_outcome(outcomes[2 * k], outcomes[2 * k + 1]), sc.outcome_levels[k]).launches += 1;
+  sc.outcome_levels.clear();
   for (uint32_t c : counts)
     if (s == STB_OK && c >= IDX_MASK) s = t.fail(STB_ERR_INDEX_CEILING, "a layer has 2^29-1 or more unique items; the pointer format cannot index it");
   if (s != STB_OK) {

@@ -26,19 +26,24 @@ void Ctx::flush_profile() {
   for (auto& p : pending) {
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, p.a, p.b) == cudaSuccess) {
-      const std::string name = p.level >= 0 ? std::string(p.name) + "@L" + std::to_string(p.level) : std::string(p.name);
-      auto it = acc.find(name);
-      if (it == acc.end()) {
-        acc_order.push_back(name);
-        it = acc.emplace(name, Acc{}).first;
-      }
-      it->second.ms += ms;
-      it->second.launches += 1;
+      Acc& a = account(p.name, p.level);
+      a.ms += ms;
+      a.launches += 1;
     }
     event_pool.push_back(p.a);
     event_pool.push_back(p.b);
   }
   pending.clear();
+}
+
+Ctx::Acc& Ctx::account(const char* name, int level) {
+  const std::string key = level >= 0 ? std::string(name) + "@L" + std::to_string(level) : std::string(name);
+  auto it = acc.find(key);
+  if (it == acc.end()) {
+    acc_order.push_back(key);
+    it = acc.emplace(key, Acc{}).first;
+  }
+  return it->second;
 }
 
 cudaError_t Ctx::copy_lane(size_t events) {

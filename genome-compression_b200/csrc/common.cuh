@@ -348,6 +348,7 @@ struct Ctx {
   }
   cudaEvent_t get_event();
   void flush_profile();  // synchronises and folds pending events into acc
+  Acc& account(const char* name, int level);  // the class "name" (level >= 0: "name@L<level>") in acc
   // a second stream for chunked host-to-device copies that later work on `stream` waits for chunk by chunk
   cudaStream_t copy_stream = nullptr;
   std::vector<cudaEvent_t> copy_events;

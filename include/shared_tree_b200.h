@@ -143,7 +143,15 @@ uint64_t stb_kernel_launches(void);
 int stb_profile_enable(stb_tree* tree, int on);
 int stb_profile_reset(stb_tree* tree);
 /* Fills names[i] (static strings), total_ms[i], launches[i] for up to cap kernel
- * classes; *count receives the number of classes. */
+ * classes; *count receives the number of classes.
+ * Besides the kernels, five classes with total_ms = 0 count the on-chip (bucketed) node levels of the
+ * builds profiled, one per level, by what that level's deduplication came to:
+ *   dedup_on_chip              every final bucket fitted its region
+ *   dedup_exact                a final bucket outgrew its region: the exact-size second pass ran
+ *   dedup_chunked              ... and a final bucket of more than 3072 records was walked in chunks
+ *   dedup_fallback_first_pass  a first-pass bucket overflowed: the level went through the table in HBM
+ *   dedup_fallback_distinct    a chunked bucket held more than 4096 distinct keys: the same fallback
+ * With the option profile_levels they carry "@L<level>" like the kernels. */
 int stb_profile_read(stb_tree* tree, const char** names, double* total_ms, uint64_t* launches,
                      uint64_t cap, uint64_t* count);
 
