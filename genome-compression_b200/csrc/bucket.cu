@@ -24,6 +24,7 @@
 // A bucket that outgrows its region raises *overflow; the dedup kernel then does nothing and
 // build.cu re-runs the level through the hash table in HBM.
 #include "bucket.cuh"
+#include "scan.cuh"
 
 namespace stb {
 
@@ -89,9 +90,9 @@ partition_tile(const uint32_t bx, const uint32_t by, const uint32_t* __restrict_
   uint32_t* loff = hist + PT_MAX_BUCKETS;
   uint32_t* goff = loff + PT_MAX_BUCKETS;
   uint16_t* sdig = reinterpret_cast<uint16_t*>(goff + PT_MAX_BUCKETS);
-  __shared__ uint32_t warp_sum[PT_WARPS];
+  __shared__ uint32_t warp_totals[PT_WARPS];
 
-  const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t tid = threadIdx.x, lane = tid & 31;
   const uint32_t nb = 1u << bits;
   uint32_t count;
   const uint32_t first = bx * PT_TILE;
@@ -247,18 +248,9 @@ partition_tile(const uint32_t bx, const uint32_t by, const uint32_t* __restrict_
   // exclusive scan of the tile's bucket counts; one global reservation per bucket
   {
     const uint32_t c = tid < nb ? hist[tid] : 0u;
-    uint32_t x = c;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
+    const uint32_t before = block_exclusive_sum<PT_THREADS>(c, warp_totals);
     if (tid < nb) {
-      uint32_t before = 0;
-      for (uint32_t w = 0; w < warp; ++w) before += warp_sum[w];
-      loff[tid] = before + x - c;
+      loff[tid] = before;
       uint32_t g = 0;
       if (c) {
         const uint32_t bucket = FROM_CHILDREN ? tid : (((by / segs) << bits) | tid);
@@ -331,33 +323,9 @@ partition_leaves_kernel(LeafFinish leaf, uint32_t n_cur, uint32_t n_next, unsign
 __global__ void __launch_bounds__(1024) exact_offsets_kernel(uint32_t* __restrict__ count2, uint32_t nb, uint32_t* __restrict__ off,
                                                               const uint32_t* __restrict__ overflow) {
   if (!exact_pass_wanted(overflow)) return;
-  __shared__ uint32_t warp_sum[32];
-  __shared__ uint32_t carry;
-  const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry = 0u;
-  __syncthreads();
-  for (uint32_t i0 = 0; i0 < nb; i0 += 1024) {
-    const uint32_t i = i0 + tid;
-    const uint32_t c = i < nb ? count2[i] : 0u;
-    uint32_t x = c;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    uint32_t before = carry;
-    for (uint32_t w = 0; w < warp; ++w) before += warp_sum[w];
-    if (i < nb) {
-      off[i] = before + x - c;
-      count2[i] = 0u;
-    }
-    __syncthreads();
-    if (tid == 1023) carry = before + x;
-    __syncthreads();
-  }
-  if (tid == 0) off[nb] = carry;
+  const uint32_t total = cta_exclusive_scan(count2, off, nb);
+  for (uint32_t i = threadIdx.x; i < nb; i += 1024) count2[i] = 0u;  // each thread clears the counts it has read
+  if (threadIdx.x == 0) off[nb] = total;
 }
 
 // the second pass again, into the exact-size regions; a grid that fits the machine walks the tiles, so the

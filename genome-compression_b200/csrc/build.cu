@@ -415,12 +415,7 @@ small_levels_kernel(const uint32_t* __restrict__ cur_in, uint32_t n_cur, SmallOu
     __syncthreads();
     if (warp == 0) {
       const uint32_t v = warp_cnt[lane];
-      uint32_t x = v;
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-        if (lane >= d) x += y;
-      }
+      const uint32_t x = warp_inclusive_sum(v);
       warp_cnt[lane] = x - v;
       if (lane == 31) counts[level] = x;
     }

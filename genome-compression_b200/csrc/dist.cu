@@ -8,6 +8,8 @@
 #include <algorithm>
 
 #include "dist.cuh"
+#include "level.cuh"
+#include "scan.cuh"
 
 namespace stb {
 
@@ -36,44 +38,6 @@ partition_hist_kernel(const void* __restrict__ items, uint64_t n_items, uint64_t
   }
   __syncthreads();
   if (threadIdx.x < world) hist[threadIdx.x * nblocks + blockIdx.x] = cnt[threadIdx.x];
-}
-
-// one CTA per owner: exclusive scan of its row + row total
-__global__ void __launch_bounds__(1024) rowscan_kernel(uint32_t* __restrict__ hist, uint32_t nblocks, uint32_t* __restrict__ row_total) {
-  __shared__ uint32_t warp_sum[32];
-  __shared__ uint32_t carry_s;
-  uint32_t* row = hist + (size_t)blockIdx.x * nblocks;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) carry_s = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < nblocks; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const uint32_t v = i < nblocks ? row[i] : 0u;
-    uint32_t x = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      uint32_t w = warp_sum[lane];
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, w, d);
-        if (lane >= d) w += y;
-      }
-      warp_sum[lane] = w;
-    }
-    __syncthreads();
-    const uint32_t before = carry_s + (warp ? warp_sum[warp - 1] : 0u) + x - v;
-    if (i < nblocks) row[i] = before;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry_s = before + v;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) row_total[blockIdx.x] = carry_s;
 }
 
 template <int KIND>
@@ -177,86 +141,31 @@ owner_answer_kernel(const uint32_t* __restrict__ gpos, uint32_t n, const Slot* t
 // per-CTA popcount of 1024 words
 __global__ void __launch_bounds__(256)
 popc_blocks_kernel(const uint32_t* __restrict__ bitmap, uint64_t n_words, uint32_t* __restrict__ block_sum) {
-  __shared__ uint32_t warp_sum[8];
+  __shared__ uint32_t warp_totals[8];
   uint32_t c = 0;
 #pragma unroll
   for (int it = 0; it < 4; ++it) {
     const uint64_t w = (uint64_t)blockIdx.x * 1024 + it * 256 + threadIdx.x;
     if (w < n_words) c += __popc(bitmap[w]);
   }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
-  if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = c;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t t = 0;
-    for (int w = 0; w < 8; ++w) t += warp_sum[w];
-    block_sum[blockIdx.x] = t;
-  }
-}
-
-__global__ void __launch_bounds__(1024) scan_u32_kernel(uint32_t* __restrict__ v, uint32_t n, uint32_t* __restrict__ total_out) {
-  __shared__ uint32_t warp_sum[32];
-  __shared__ uint32_t carry_s;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) carry_s = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const uint32_t x0 = i < n ? v[i] : 0u;
-    uint32_t x = x0;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      uint32_t w = warp_sum[lane];
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, w, d);
-        if (lane >= d) w += y;
-      }
-      warp_sum[lane] = w;
-    }
-    __syncthreads();
-    const uint32_t before = carry_s + (warp ? warp_sum[warp - 1] : 0u) + x - x0;
-    if (i < n) v[i] = before;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry_s = before + x0;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *total_out = carry_s;
+  uint32_t total;
+  block_exclusive_sum<256>(c, warp_totals, &total);
+  if (threadIdx.x == 0) block_sum[blockIdx.x] = total;
 }
 
 // word_prefix[w] = number of set bits in words [0, w); one CTA per 1024 words (sequential in 4 rows)
 __global__ void __launch_bounds__(256)
 word_prefix_kernel(const uint32_t* __restrict__ bitmap, uint64_t n_words, const uint32_t* __restrict__ block_prefix,
                    uint32_t* __restrict__ word_prefix) {
-  __shared__ uint32_t warp_sum[8];
-  __shared__ uint32_t carry_s;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) carry_s = block_prefix[blockIdx.x];
-  __syncthreads();
+  __shared__ uint32_t warp_totals[8];
+  uint32_t carry = block_prefix[blockIdx.x];
   for (int it = 0; it < 4; ++it) {
     const uint64_t w = (uint64_t)blockIdx.x * 1024 + it * 256 + threadIdx.x;
-    const uint32_t v = w < n_words ? __popc(bitmap[w]) : 0u;
-    uint32_t x = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    uint32_t before = carry_s;
-    for (uint32_t k = 0; k < warp; ++k) before += warp_sum[k];
-    if (w < n_words) word_prefix[w] = before + x - v;
-    __syncthreads();
-    if (threadIdx.x == 255) carry_s = before + x;
-    __syncthreads();
+    uint32_t row_total;
+    const uint32_t before = block_exclusive_sum<256>(w < n_words ? __popc(bitmap[w]) : 0u, warp_totals, &row_total);
+    if (w < n_words) word_prefix[w] = carry + before;
+    carry += row_total;
+    __syncthreads();  // the next row writes warp_totals again
   }
 }
 
@@ -277,14 +186,6 @@ finish_rest_kernel(uint64_t n_pos, uint64_t gpos0, const uint32_t* __restrict__ 
 constexpr uint32_t DIRECT_EMPTY = 0x7f7f7f7fu;  // > any position, positive as int32 (all-reduce MIN)
 
 __global__ void __launch_bounds__(256)
-direct_mark_kernel(const uint32_t* __restrict__ table, uint32_t entries, uint32_t* __restrict__ bitmap) {
-  const uint32_t s = blockIdx.x * 256 + threadIdx.x;
-  if (s >= entries) return;
-  const uint32_t mp = __ldg(table + s);
-  if (mp < DIRECT_EMPTY) atomicOr(bitmap + (mp >> 5), 1u << (mp & 31));
-}
-
-__global__ void __launch_bounds__(256)
 direct_ids_kernel(const uint32_t* __restrict__ table, uint32_t entries, const uint32_t* __restrict__ bitmap,
                   const uint32_t* __restrict__ word_prefix, uint64_t n_bits, uint64_t n_words, int S, uint32_t* __restrict__ ids,
                   unsigned long long* __restrict__ leaves_out) {
@@ -295,14 +196,6 @@ direct_ids_kernel(const uint32_t* __restrict__ table, uint32_t entries, const ui
   const uint32_t id = rank_of(bitmap, word_prefix, n_bits, n_words, mp);
   ids[s] = id;
   leaves_out[id] = leaf_from_2bit(s, S);
-}
-
-__global__ void __launch_bounds__(256)
-direct_resolve_kernel(const uint32_t* __restrict__ tmp, uint64_t n, const uint32_t* __restrict__ ids, uint32_t* __restrict__ pointers) {
-  const uint64_t i = (uint64_t)blockIdx.x * 256 + threadIdx.x;
-  if (i >= n) return;
-  const uint32_t t = __ldg(tmp + i);
-  pointers[i] = finish_pointer(__ldg(ids + (t & IDX_MASK)), t & ~IDX_MASK);
 }
 
 }  // namespace stb
@@ -340,7 +233,7 @@ int stb_dist_partition(stb_tree* ctx, int kind, const void* items_dev, uint64_t 
   }
   {
     Launch l(t, "dist_rowscan");
-    rowscan_kernel<<<world, 1024, 0, st>>>(hist.ptr, nblocks, counts_dev);
+    exclusive_scan_rows_kernel<<<world, 1024, 0, st>>>(hist.ptr, nblocks, counts_dev);  // one row per owner
   }
   {
     Launch l(t, "dist_partition_scatter");
@@ -409,7 +302,7 @@ int stb_dist_rank_index(stb_tree* ctx, const uint32_t* bitmap_dev, uint64_t n_wo
   }
   {
     Launch l(t, "dist_scan");
-    scan_u32_kernel<<<1, 1024, 0, st>>>(scratch_dev, nblocks, word_prefix_dev + n_words);
+    exclusive_scan_rows_kernel<<<1, 1024, 0, st>>>(scratch_dev, nblocks, word_prefix_dev + n_words);
   }
   {
     Launch l(t, "dist_word_prefix");
@@ -461,7 +354,7 @@ int stb_dist_leaf_direct_finish(stb_tree* ctx, const uint32_t* table_dev, uint64
   const uint64_t n_words = ceil_div(n_level_positions, 32);
   {
     Launch l(t, "dist_direct_mark");
-    direct_mark_kernel<<<(unsigned)ceil_div(entries, 256), 256, 0, st>>>(table_dev, entries, bitmap_dev);
+    mark_first_kernel<<<(unsigned)ceil_div(entries, 256), 256, 0, st>>>(table_dev, entries, bitmap_dev);
   }
   STB_TRY(stb_dist_rank_index(ctx, bitmap_dev, n_words, word_prefix_dev, scratch_dev));
   {
@@ -471,7 +364,7 @@ int stb_dist_leaf_direct_finish(stb_tree* ctx, const uint32_t* table_dev, uint64
   }
   if (n_local) {
     Launch l(t, "dist_direct_resolve");
-    direct_resolve_kernel<<<(unsigned)ceil_div(n_local, 256), 256, 0, st>>>(tmp_dev, n_local, ids_dev, pointers_dev);
+    finish_leaves_kernel<<<(unsigned)ceil_div(n_local, 256), 256, 0, st>>>(tmp_dev, n_local, ids_dev, pointers_dev);
   }
   STB_CUDA(t, cudaGetLastError());
   return STB_OK;

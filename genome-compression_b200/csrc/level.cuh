@@ -3,6 +3,7 @@
 #pragma once
 
 #include "common.cuh"
+#include "scan.cuh"
 
 namespace stb {
 
@@ -45,12 +46,7 @@ __device__ __forceinline__ void tile_prefix(const uint32_t* __restrict__ bitmask
   __syncthreads();
   if (warp == 0) {
     const uint32_t v = word_pref[lane];
-    uint32_t x = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
+    const uint32_t x = warp_inclusive_sum(v);
     word_pref[lane] = x - v;
     if (lane == 31) word_pref[32] = x;
   }
@@ -105,9 +101,7 @@ constexpr uint32_t CHUNK_TILES = 256;
 __device__ __forceinline__ void count_tile(const uint32_t* __restrict__ bitmask, uint32_t tile, uint32_t rel, uint32_t* __restrict__ blockcnt,
                                            uint32_t* __restrict__ chunkcnt) {
   const uint32_t lane = threadIdx.x & 31;
-  uint32_t c = __popc(bitmask[(uint64_t)tile * (LVL_TILE / 32) + lane]);
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) c += __shfl_xor_sync(0xffffffffu, c, d);
+  const uint32_t c = warp_sum((uint32_t)__popc(bitmask[(uint64_t)tile * (LVL_TILE / 32) + lane]));
   if (lane == 0) {
     blockcnt[rel] = c;
     if (c) atomicAdd(chunkcnt + rel / CHUNK_TILES, c);
@@ -131,8 +125,7 @@ __device__ __forceinline__ uint32_t tile_base(uint32_t rel, const uint32_t* __re
   const uint32_t chunk = rel / CHUNK_TILES, in_chunk = chunk * CHUNK_TILES + threadIdx.x;
   uint32_t part = in_chunk < rel ? blockcnt[in_chunk] : 0u;
   for (uint32_t i = threadIdx.x; i < chunk; i += LVL_THREADS) part += chunkcnt[i];
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) part += __shfl_xor_sync(0xffffffffu, part, d);
+  part = warp_sum(part);
   if (lane == 0) red[warp] = part;
   __syncthreads();
   uint32_t base = 0;
@@ -161,6 +154,27 @@ assign_kernel(uint32_t* __restrict__ tmp, uint32_t n, LevelTable tab, const uint
   tile_prefix(bitmask, block, n, words, word_pref);
   if (rel == gridDim.x - 1 && threadIdx.x == 0) *total_out = base + word_pref[32];
   assign_tile<MODE>(block, base, words, word_pref, tmp, n, tab, uniq, S, children, n_children, id_offset ? *id_offset : 0u);
+}
+
+// Leaf level of the sharded builds (shard.cu, dist.cu), where the leaf table is replicated: minpos[c] is
+// the first global position of code c.  Sets the bit of every such position.  An unused entry holds
+// 0xffffffff (shard.cu) or 0x7f7f7f7f (dist.cu); positions are below 2^30, so both fail the test.
+static __global__ void __launch_bounds__(256)
+mark_first_kernel(const uint32_t* __restrict__ minpos, uint32_t entries, uint32_t* __restrict__ bits) {
+  const uint32_t c = blockIdx.x * 256 + threadIdx.x;
+  if (c >= entries) return;
+  const uint32_t q = __ldg(minpos + c);
+  if (q < 0x7f7f7f7fu) atomicOr(bits + (q >> 5), 1u << (q & 31));
+}
+
+// ... and finishes a rank's leaf pointers from the id table: tmp[i] = code | flags, as the leaf insert left
+// it.  tmp == pointers finishes them in place.
+static __global__ void __launch_bounds__(256)
+finish_leaves_kernel(const uint32_t* tmp, uint64_t n, const uint32_t* __restrict__ ids, uint32_t* pointers) {
+  const uint64_t i = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t t = tmp[i];
+  pointers[i] = finish_pointer(__ldg(ids + (t & IDX_MASK)), t & ~IDX_MASK);
 }
 
 }  // namespace stb

@@ -13,6 +13,7 @@
 #include <algorithm>
 #include <cstring>
 
+#include "scan.cuh"
 #include "staging.cuh"
 #include "tree.h"
 
@@ -45,7 +46,7 @@ __host__ __device__ __forceinline__ uint32_t ptr_encode(uint32_t raw, uint8_t* o
 
 __global__ void __launch_bounds__(SER_THREADS)
 node_tile_bytes_kernel(const uint2* __restrict__ nodes, uint32_t n, unsigned long long* __restrict__ tile_bytes) {
-  __shared__ uint32_t sm[8];
+  __shared__ uint32_t sm[SER_THREADS / 32];
   uint32_t mine = 0;
   const uint32_t first = blockIdx.x * SER_TILE + threadIdx.x * SER_PER_THREAD;
 #pragma unroll
@@ -55,52 +56,14 @@ node_tile_bytes_kernel(const uint2* __restrict__ nodes, uint32_t n, unsigned lon
       mine += ptr_len(nd.x) + ptr_len(nd.y);
     }
   uint32_t total;
-  block_exclusive_sum_256(mine, sm, &total);
+  block_exclusive_sum<SER_THREADS>(mine, sm, &total);
   if (threadIdx.x == 0) tile_bytes[blockIdx.x] = total;
-}
-
-// exclusive scan (single CTA) of 64-bit tile sizes, in place; total -> *total_out
-__global__ void __launch_bounds__(1024)
-scan_u64_kernel(unsigned long long* __restrict__ v, uint32_t n, unsigned long long* __restrict__ total_out) {
-  __shared__ unsigned long long warp_sum[32];
-  __shared__ unsigned long long carry_s;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) carry_s = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < n; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const unsigned long long x0 = i < n ? v[i] : 0ull;
-    unsigned long long x = x0;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const unsigned long long y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      unsigned long long w = warp_sum[lane];
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const unsigned long long y = __shfl_up_sync(0xffffffffu, w, d);
-        if (lane >= d) w += y;
-      }
-      warp_sum[lane] = w;
-    }
-    __syncthreads();
-    const unsigned long long before = carry_s + (warp ? warp_sum[warp - 1] : 0ull) + x - x0;
-    if (i < n) v[i] = before;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry_s = before + x0;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *total_out = carry_s;
 }
 
 __global__ void __launch_bounds__(SER_THREADS)
 emit_nodes_kernel(const uint2* __restrict__ nodes, uint32_t n, const unsigned long long* __restrict__ tile_off,
                   uint8_t* __restrict__ out, unsigned long long layer_base) {
-  __shared__ uint32_t sm[8];
+  __shared__ uint32_t sm[SER_THREADS / 32];
   __shared__ __align__(16) uint8_t stage[SER_TILE * 8 + 16];
   const unsigned long long dst = layer_base + tile_off[blockIdx.x];
   const uint32_t shift = (uint32_t)(dst & 3ull);
@@ -116,7 +79,7 @@ emit_nodes_kernel(const uint2* __restrict__ nodes, uint32_t n, const unsigned lo
     }
   }
   uint32_t total;
-  uint32_t o = shift + block_exclusive_sum_256(mine, sm, &total);
+  uint32_t o = shift + block_exclusive_sum<SER_THREADS>(mine, sm, &total);
 #pragma unroll
   for (int j = 0; j < SER_PER_THREAD; ++j)
     if (first + j < n) {
@@ -181,7 +144,7 @@ int stream_plan(Tree& t) {
     }
     {
       Launch l(t, "scan_tile_bytes");
-      scan_u64_kernel<<<1, 1024, 0, st>>>(t.layer_tile_off[k].ptr, tiles, totals.ptr + k);
+      exclusive_scan_rows_kernel<<<1, 1024, 0, st>>>(t.layer_tile_off[k].ptr, tiles, totals.ptr + k);
     }
   }
   std::vector<unsigned long long> h(L);

@@ -327,38 +327,18 @@ struct LocalComm : Comm {
 
 // ---- kernels of the sharded level loop -----------------------------------------------------------
 
-// leaf level: the bit of every code's first (global) position
-__global__ void __launch_bounds__(256) leaf_mark_first_kernel(const uint32_t* __restrict__ minpos, uint32_t entries, uint32_t* __restrict__ bits) {
-  const uint32_t c = blockIdx.x * 256 + threadIdx.x;
-  if (c >= entries) return;
-  const uint32_t q = minpos[c];
-  if (q != 0xffffffffu) atomicOr(bits + (q >> 5), 1u << (q & 31));
-}
-
 // exclusive prefix of the tile counts (tilecnt, in place); one CTA per chunk of CHUNK_TILES tiles
 __global__ void __launch_bounds__(LVL_THREADS) tile_prefix_kernel(uint32_t* __restrict__ tilecnt, const uint32_t* __restrict__ chunkcnt, uint32_t tiles) {
-  __shared__ uint32_t warp_sum[LVL_THREADS / 32];
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  __shared__ uint32_t warp_totals[LVL_THREADS / 32], chunks_before[LVL_THREADS / 32];
   const uint32_t t = blockIdx.x * CHUNK_TILES + threadIdx.x;
-  uint32_t before = 0;
-  for (uint32_t i = threadIdx.x; i < blockIdx.x; i += LVL_THREADS) before += chunkcnt[i];
+  uint32_t part = 0;
+  for (uint32_t i = threadIdx.x; i < blockIdx.x; i += LVL_THREADS) part += chunkcnt[i];
+  part = warp_sum(part);
+  if ((threadIdx.x & 31) == 0) chunks_before[threadIdx.x >> 5] = part;
+  uint32_t before = block_exclusive_sum<LVL_THREADS>(t < tiles ? tilecnt[t] : 0u, warp_totals);  // its barrier publishes chunks_before
 #pragma unroll
-  for (int d = 16; d > 0; d >>= 1) before += __shfl_xor_sync(0xffffffffu, before, d);
-  const uint32_t v = t < tiles ? tilecnt[t] : 0u;
-  uint32_t x = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-    if (lane >= d) x += y;
-  }
-  if (lane == 31) warp_sum[warp] = x;
-  __shared__ uint32_t chunk_before[LVL_THREADS / 32];
-  if (lane == 0) chunk_before[warp] = before;
-  __syncthreads();
-  uint32_t base = 0;
-  for (int w = 0; w < LVL_THREADS / 32; ++w) base += chunk_before[w];
-  for (uint32_t w = 0; w < warp; ++w) base += warp_sum[w];
-  if (t < tiles) tilecnt[t] = base + x - v;
+  for (int w = 0; w < LVL_THREADS / 32; ++w) before += chunks_before[w];
+  if (t < tiles) tilecnt[t] = before;
 }
 
 // leaf ids: id(code) = rank of the code's first position; the leaf table in id order
@@ -374,14 +354,6 @@ leaf_ids_kernel(const uint32_t* __restrict__ minpos, uint32_t entries, const uin
   for (uint32_t i = w0; i < w; ++i) id += __popc(bits[i]);
   ids[c] = id;
   leaves[id] = leaf_from_2bit(c, S);
-}
-
-// local leaf pointers from the id table (tmp = canonical code | flags, as leaf_insert left it)
-__global__ void __launch_bounds__(256) leaf_pointers_kernel(uint32_t* __restrict__ tmp, uint32_t n, const uint32_t* __restrict__ ids) {
-  const uint32_t i = blockIdx.x * 256 + threadIdx.x;
-  if (i >= n) return;
-  const uint32_t t = tmp[i];
-  tmp[i] = finish_pointer(__ldcg(ids + (t & IDX_MASK)), t & ~IDX_MASK);
 }
 
 // The home rank applies the answers about its positions: it reads the list every owner kept for it
@@ -431,18 +403,12 @@ apply_answers_kernel(PeerHome home, uint32_t world, uint32_t* __restrict__ aux, 
 
 // local number of first occurrences = sum of the chunk totals
 __global__ void __launch_bounds__(256) sum_chunks_kernel(const uint32_t* __restrict__ chunkcnt, uint32_t chunks, uint32_t* __restrict__ out) {
-  __shared__ uint32_t red[8];
+  __shared__ uint32_t warp_totals[8];
   uint32_t s = 0;
   for (uint32_t i = threadIdx.x; i < chunks; i += 256) s += chunkcnt[i];
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) s += __shfl_xor_sync(0xffffffffu, s, d);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t t = 0;
-    for (int w = 0; w < 8; ++w) t += red[w];
-    *out = t;
-  }
+  uint32_t total;
+  block_exclusive_sum<256>(s, warp_totals, &total);
+  if (threadIdx.x == 0) *out = total;
 }
 
 // ids of this rank start after the first occurrences of the ranks before it
@@ -696,7 +662,7 @@ int shard_build(Shard& s, const char* d_body, uint64_t n_bases_total) {
     STB_CUDA(s, cudaMemsetAsync(s.leaf_bits.ptr, 0, (uint64_t)tiles * (LVL_TILE / 8), st));
     STB_CUDA(s, cudaMemsetAsync(chunkcnt, 0, (uint64_t)chunks * 4, st));
     Launch l(s, "shard_leaf_ids");
-    leaf_mark_first_kernel<<<(unsigned)ceil_div(canon_entries, 256), 256, 0, st>>>(s.dminpos.ptr, (uint32_t)canon_entries, s.leaf_bits.ptr);
+    mark_first_kernel<<<(unsigned)ceil_div(canon_entries, 256), 256, 0, st>>>(s.dminpos.ptr, (uint32_t)canon_entries, s.leaf_bits.ptr);
     count_kernel<<<(unsigned)ceil_div((uint64_t)tiles * 32, 256), 256, 0, st>>>(s.leaf_bits.ptr, 0u, tiles, s.tilecnt.ptr, chunkcnt);
     sum_chunks_kernel<<<1, 256, 0, st>>>(chunkcnt, chunks, s.totals_all.ptr);  // level 0 total: the same on every rank
     tile_prefix_kernel<<<chunks, LVL_THREADS, 0, st>>>(s.tilecnt.ptr, chunkcnt, tiles);
@@ -707,7 +673,7 @@ int shard_build(Shard& s, const char* d_body, uint64_t n_bases_total) {
   const bool fuse_leaf = L > 1;
   if (n_local && !fuse_leaf) {
     Launch l(s, "shard_leaf_pointers");
-    leaf_pointers_kernel<<<(unsigned)ceil_div(n_local, 256), 256, 0, st>>>(ptr_cur, (uint32_t)n_local, s.dids.ptr);
+    finish_leaves_kernel<<<(unsigned)ceil_div(n_local, 256), 256, 0, st>>>(ptr_cur, n_local, s.dids.ptr, ptr_cur);
   }
 
   // ---- sharded node levels ----

@@ -15,6 +15,7 @@
 // straight into newpos[].
 #include <algorithm>
 
+#include "scan.cuh"
 #include "tree.h"
 
 namespace stb {
@@ -91,45 +92,6 @@ radix_hist_kernel(const uint32_t* __restrict__ keys, uint32_t n, uint32_t maxf, 
   hist[threadIdx.x * nblocks + blockIdx.x] = bins[threadIdx.x];
 }
 
-// One CTA per digit: exclusive scan of its row (in place) + row total.
-__global__ void __launch_bounds__(1024)
-radix_rowscan_kernel(uint32_t* __restrict__ hist, uint32_t nblocks, uint32_t* __restrict__ row_total) {
-  __shared__ uint32_t warp_sum[32];
-  __shared__ uint32_t carry_s;
-  uint32_t* row = hist + (size_t)blockIdx.x * nblocks;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (threadIdx.x == 0) carry_s = 0;
-  __syncthreads();
-  for (uint32_t base = 0; base < nblocks; base += 1024) {
-    const uint32_t i = base + threadIdx.x;
-    const uint32_t v = i < nblocks ? row[i] : 0u;
-    uint32_t x = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) warp_sum[warp] = x;
-    __syncthreads();
-    if (warp == 0) {
-      uint32_t w = warp_sum[lane];
-#pragma unroll
-      for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t y = __shfl_up_sync(0xffffffffu, w, d);
-        if (lane >= d) w += y;
-      }
-      warp_sum[lane] = w;
-    }
-    __syncthreads();
-    const uint32_t before = carry_s + (warp ? warp_sum[warp - 1] : 0u) + x - v;
-    if (i < nblocks) row[i] = before;
-    __syncthreads();
-    if (threadIdx.x == 1023) carry_s = before + v;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) row_total[blockIdx.x] = carry_s;
-}
-
 // Scatter pass.  FIRST: values are the implicit identity.  LAST: instead of moving the
 // pair, publish the destination rank: newpos[value] = rank.
 template <bool FIRST, bool LAST>
@@ -142,21 +104,8 @@ radix_scatter_kernel(const uint32_t* __restrict__ keys_in, const uint32_t* __res
   __shared__ uint32_t warp_cnt[RS_WARPS][256];    // per-warp counts, then running offsets
   __shared__ uint32_t scan_tmp[RS_WARPS];
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  // exclusive scan of the 256 row totals (8 warps x 32 lanes)
-  {
-    const uint32_t v = row_total[threadIdx.x];
-    uint32_t x = v;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-      if (lane >= d) x += y;
-    }
-    if (lane == 31) scan_tmp[warp] = x;
-    __syncthreads();
-    uint32_t before = 0;
-    for (uint32_t w = 0; w < warp; ++w) before += scan_tmp[w];
-    digit_base[threadIdx.x] = before + x - v + hist[threadIdx.x * nblocks + blockIdx.x];
-  }
+  // exclusive scan of the 256 row totals
+  digit_base[threadIdx.x] = block_exclusive_sum<RS_THREADS>(row_total[threadIdx.x], scan_tmp) + hist[threadIdx.x * nblocks + blockIdx.x];
 #pragma unroll
   for (int w = 0; w < RS_WARPS; ++w) warp_cnt[w][threadIdx.x] = 0;
   __syncthreads();
@@ -375,8 +324,8 @@ int sort_tree(Tree& t) {
         radix_hist_kernel<<<nblocks, RS_THREADS, 0, st>>>(kin, n, maxf[c], shift, nblocks, hist);
       }
       {
-        Launch l(t, "radix_rowscan");
-        radix_rowscan_kernel<<<256, 1024, 0, st>>>(hist, nblocks, row_total);
+        Launch l(t, "radix_rowscan");  // one row per digit
+        exclusive_scan_rows_kernel<<<256, 1024, 0, st>>>(hist, nblocks, row_total);
       }
       {
         Launch l(t, "radix_scatter");

@@ -30,27 +30,4 @@ __device__ __forceinline__ void copy_out_staged(char* dst_aligned, const uint8_t
   }
 }
 
-// Block-wide exclusive sum for 256-thread CTAs; returns the exclusive prefix, total in *total.
-__device__ __forceinline__ uint32_t block_exclusive_sum_256(uint32_t v, uint32_t* smem_warp8, uint32_t* total) {
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  uint32_t x = v;
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) {
-    const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
-    if (lane >= d) x += y;
-  }
-  if (lane == 31) smem_warp8[warp] = x;
-  __syncthreads();
-  uint32_t before = 0, tot = 0;
-#pragma unroll
-  for (uint32_t w = 0; w < 8; ++w) {
-    const uint32_t s = smem_warp8[w];
-    if (w < warp) before += s;
-    tot += s;
-  }
-  *total = tot;
-  __syncthreads();
-  return before + x - v;
-}
-
 }  // namespace stb

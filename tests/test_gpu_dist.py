@@ -89,6 +89,26 @@ def test_virtual_ranks_synthetic_large(stb):
         assert full.serialize() == single.serialize()
 
 
+def test_rank_index_past_1024_blocks(stb):
+    """More than 1024 blocks of 1024 words: the scan of the block sums carries across its
+    1024-element rounds."""
+    import torch
+    from genome_compression_b200.dist import CudaStages
+
+    n_words = (1 << 21) + 777
+    bitmap = np.random.default_rng(21).integers(0, 1 << 32, size=n_words, dtype=np.uint64).astype(np.uint32)
+    stages = CudaStages(stb, 12, 0)
+    bitmap_dev = torch.from_numpy(bitmap.view(np.int32)).cuda()
+    word_prefix = torch.empty(n_words + 1, dtype=torch.int32, device="cuda")
+    scratch = torch.empty(-(-n_words // 1024) + 1, dtype=torch.int32, device="cuda")
+    torch.cuda.synchronize()
+    stages.rank_index(bitmap_dev, n_words, word_prefix, scratch)
+    torch.cuda.synchronize()
+    popcount = np.unpackbits(bitmap.view(np.uint8)).reshape(n_words, 32).sum(axis=1)
+    want = np.concatenate([[0], np.cumsum(popcount)]).astype(np.uint32)
+    assert np.array_equal(word_prefix.cpu().numpy().view(np.uint32), want)
+
+
 def test_nccl_two_ranks(stb):
     import torch
     if torch.cuda.device_count() < 2:
