@@ -19,6 +19,14 @@
 //     resolve  later occurrences: slot -> min-position -> the first occurrence's
 //              finished pointer -> id                          [random reads]
 //
+//   node levels built one kernel at a time (option fused_resolve, default on):
+//     count        tile popcounts + each bitmap word's prefix inside its tile
+//     tile_bases   absolute first-occurrence count before every tile
+//     assign_resolve  first occurrences as in assign; a later occurrence takes the
+//              rank of its first occurrence from that rank directory (bitmap, word
+//              prefixes, tile bases: L2-sized), so no second pass reads the
+//              first occurrence's pointer                      [coalesced + L2]
+//
 // IDs are first-occurrence ranks in position order, independent of which thread won
 // which atomic, so the result equals the reference's sequential emplace order.
 #include <cooperative_groups.h>
@@ -352,6 +360,45 @@ resolve_kernel(const uint32_t* aux, uint32_t* out, uint32_t n, LevelTable tab, c
   }
 }
 
+// A node level with its rank directory (RankDir, level.cuh) in one pass: first occurrences as in
+// assign_tile, later occurrences as in resolve_kernel<RESOLVE_TABLE>, except that the id of the first
+// occurrence q is q's rank, not read from out[q] - so nothing here reads a pointer this launch writes.
+// Bitmap words, word prefixes and tile bases are read-only for the whole launch (ld.global.nc).
+__global__ void __launch_bounds__(LVL_THREADS)
+assign_resolve_kernel(const uint32_t* __restrict__ aux, uint32_t* __restrict__ out, uint32_t n, LevelTable tab, const uint32_t* __restrict__ bitmask,
+                      RankDir dir, uint32_t* __restrict__ multi_bits, const uint32_t* __restrict__ firstpos_unless, void* __restrict__ uniq,
+                      const uint32_t* __restrict__ children, uint32_t n_children) {
+  const uint32_t lane = threadIdx.x & 31;
+  const bool firstpos = firstpos_unless && *firstpos_unless == 0u;
+  const uint32_t base = __ldg(dir.tilebase + blockIdx.x);
+#pragma unroll
+  for (int it = 0; it < LVL_ITERS; ++it) {
+    const uint32_t p = blockIdx.x * LVL_TILE + it * LVL_THREADS + threadIdx.x;
+    if (p >= n) continue;
+    const uint32_t word = __ldg(bitmask + (p >> 5));
+    if ((word >> lane) & 1u) {
+      const uint32_t rank = base + __ldg(dir.wpref + (p >> 5)) + __popc(word & ((1u << lane) - 1u));
+      assign_position<MODE_NODE>(p, rank, out, tab, uniq, 0, children, n_children);
+      continue;
+    }
+    const uint32_t t = aux[p];
+    uint32_t q = t & IDX_MASK;
+    if (!firstpos) {
+      q = __ldcg(&tab.slots[q].minpos);
+      // test before set: the positions of an N run (or of any long run) all name the same first occurrence
+      if (multi_bits && !((__ldcg(multi_bits + (q >> 5)) >> (q & 31u)) & 1u)) atomicOr(multi_bits + (q >> 5), 1u << (q & 31));
+    }
+    uint32_t qword = __ldg(bitmask + (q >> 5));
+    if (firstpos && p - q < COLLAPSE_WINDOW && !((qword >> (q & 31u)) & 1u)) {
+      // p repeats its predecessor and q is the head of its run (bucket.cu), itself a later occurrence
+      q = __ldcg(aux + q) & IDX_MASK;
+      qword = __ldg(bitmask + (q >> 5));
+    }
+    const uint32_t id = __ldg(dir.tilebase + q / LVL_TILE) + __ldg(dir.wpref + (q >> 5)) + __popc(qword & ((1u << (q & 31u)) - 1u));
+    out[p] = finish_pointer(id, t & ~IDX_MASK);
+  }
+}
+
 // Clears the level's bitmaps when the on-chip path gave up (the hash-table fallback starts from zero).
 __global__ void __launch_bounds__(256) bitmaps_reset_kernel(uint32_t* __restrict__ a, uint32_t* __restrict__ b, uint32_t words,
                                                             const uint32_t* __restrict__ enable) {
@@ -575,6 +622,8 @@ struct Scratch {
   DevBuf<uint32_t> ptr_a, ptr_b, aux, bitmask, counts, dminpos, dids;
   DevBuf<uint32_t> lvl_bits[2], lvl_multi[2];  // node levels: first occurrences / first occurrences that occur again, by level parity
   DevBuf<uint32_t> tilecnt;                    // first occurrences per tile, then per chunk of tiles (count_kernel)
+  DevBuf<uint16_t> wpref;                      // rank directory of the node levels (RankDir)
+  DevBuf<uint32_t> tilebase;
   DevBuf<uint32_t> leaf_done, leaf_carry;      // leaf level after a prefix: positions finished by the leaf kernel; first occurrences in the prefix
   DevBuf<Slot> side_slots;
   DevBuf<BuildFlags> flags;
@@ -657,15 +706,28 @@ TileWindow whole_level(uint64_t n, uint32_t* total) { return {0u, (uint32_t)ceil
 // count -> assign -> resolve over a window of one level whose inserts are already queued.  `aux` is
 // what the inserts left per position, `out` receives the finished pointers (the same array for the
 // leaf level); assign and resolve see positions below n_assign and n_resolve.
+// `dir` (node levels, a whole level, aux != out, n_assign == n_resolve): count (with the word
+// prefixes) -> tile bases -> assign_resolve instead.
 template <int MODE>
 int finish_level(Ctx& ctx, const TileWindow& w, const uint32_t* aux, uint32_t* out, uint32_t n_assign, uint32_t n_resolve, LevelTable tab,
                  const uint32_t* bitmask, uint32_t* tilecnt, void* uniq, const uint32_t* children = nullptr, uint32_t n_children = 0,
-                 uint32_t* multi_bits = nullptr, const uint32_t* firstpos_unless = nullptr, bool skip_resolve = false) {
+                 uint32_t* multi_bits = nullptr, const uint32_t* firstpos_unless = nullptr, bool skip_resolve = false, const RankDir* dir = nullptr) {
   uint32_t* chunkcnt = tilecnt + w.count;
   STB_CUDA(ctx, cudaMemsetAsync(chunkcnt, 0, (w.count / CHUNK_TILES + 1) * 4, ctx.stream));
   {
     Launch l(ctx, "count_firsts");
-    count_kernel<<<(unsigned)ceil_div((uint64_t)w.count * 32, 256), 256, 0, ctx.stream>>>(bitmask, w.first, w.count, tilecnt, chunkcnt);
+    count_kernel<<<(unsigned)ceil_div((uint64_t)w.count * 32, 256), 256, 0, ctx.stream>>>(bitmask, w.first, w.count, tilecnt, chunkcnt,
+                                                                                          dir ? dir->wpref : nullptr);
+  }
+  if (MODE == MODE_NODE && dir) {
+    {
+      Launch l(ctx, "tile_bases");
+      tile_bases_kernel<<<(unsigned)ceil_div(w.count, CHUNK_TILES), CHUNK_TILES, 0, ctx.stream>>>(tilecnt, chunkcnt, w.count, dir->tilebase, w.total);
+    }
+    Launch l(ctx, "assign_resolve");
+    assign_resolve_kernel<<<w.count, LVL_THREADS, 0, ctx.stream>>>(aux, out, n_assign, tab, bitmask, *dir, multi_bits, firstpos_unless, uniq, children,
+                                                                    n_children);
+    return STB_OK;
   }
   {
     Launch l(ctx, "assign_ids");
@@ -696,6 +758,8 @@ int reserve_node_workspace(Tree& t, Scratch& sc, uint64_t n_cur) {
     const uint64_t tiles = ceil_div(n_cur, LVL_TILE);
     STB_CUDA(t, sc.tilecnt.ensure(tiles + tiles / CHUNK_TILES + 2, st));
   }
+  STB_CUDA(t, sc.wpref.ensure(bitmap_words(n1), st));
+  STB_CUDA(t, sc.tilebase.ensure(ceil_div(n1, LVL_TILE), st));
   STB_CUDA(t, sc.counts.ensure(80, st));
   STB_CUDA(t, sc.root.ensure(1, st));
   STB_CUDA(t, sc.slots.ensure((uint64_t)table_cap(n1) + 1, st));
@@ -827,8 +891,10 @@ int run_node_levels(Tree& t, Scratch& sc, uint32_t* cur, uint32_t* nxt, uint64_t
       node_insert_kernel<<<pl.usable ? std::min(nb, 1184u) : nb, LVL_THREADS, 0, st>>>(cur, (uint32_t)n_cur, (uint32_t)n_next, nt, sc.aux.ptr, child_unique,
                                                                                         sc.slots.take(1), child_first, child_multi, 0u, overflow);
     }
+    const RankDir dir{sc.wpref.ptr, sc.tilebase.ptr};
     STB_TRY(finish_level<MODE_NODE>(t, whole_level(n_next, counts_dev + level), sc.aux.ptr, nxt, (uint32_t)n_next, (uint32_t)n_next, nt, first_bits,
-                                    sc.tilecnt.ptr, layer.nodes.ptr, cur, (uint32_t)n_cur, multi_bits, overflow));
+                                    sc.tilecnt.ptr, layer.nodes.ptr, cur, (uint32_t)n_cur, multi_bits, overflow, false,
+                                    t.opt.fused_resolve ? &dir : nullptr));
     std::swap(cur, nxt);
     n_cur = n_next;
     ++level;

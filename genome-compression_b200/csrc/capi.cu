@@ -167,7 +167,8 @@ static uint64_t* option_slot(Options& o, const char* name) {
   const struct { const char* name; uint64_t* slot; } table[] = {
       {"bucket_min", &o.bucket_min}, {"bucket_levels", &o.bucket_levels}, {"bucket_cap", &o.bucket_cap}, {"partition_threads", &o.partition_threads}, {"dedup_threads", &o.dedup_threads}, {"bucket_slack_permille", &o.bucket_slack_permille}, {"bucket_headroom", &o.bucket_headroom},
       {"child_filter", &o.child_filter}, {"locality", &o.locality}, {"coop_max", &o.coop_max}, {"reserve_pipeline", &o.reserve_pipeline}, {"side_table_slots", &o.side_table_slots}, {"profile_levels", &o.profile_levels},
-      {"stream_chunk_log2", &o.stream_chunk_log2}, {"stream_min_chunks", &o.stream_min_chunks}, {"leaf_prefix_log2", &o.leaf_prefix_log2}};
+      {"stream_chunk_log2", &o.stream_chunk_log2}, {"stream_min_chunks", &o.stream_min_chunks}, {"leaf_prefix_log2", &o.leaf_prefix_log2},
+      {"fused_resolve", &o.fused_resolve}};
   for (const auto& e : table)
     if (std::strcmp(e.name, name) == 0) return e.slot;
   return nullptr;

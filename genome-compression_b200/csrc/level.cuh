@@ -53,10 +53,34 @@ __device__ __forceinline__ void tile_prefix(const uint32_t* __restrict__ bitmask
   __syncthreads();
 }
 
-// First occurrences of one tile: id = rank in position order; append the item to its layer in id
-// order and emit the finished pointer.  Node items are recomputed from the child pointers
-// (coalesced) rather than fetched from a table (random).
+// The first occurrence at position p, whose id is `rank`: append its item to the layer in id order and
+// emit its finished pointer.  Node items are recomputed from the child pointers (coalesced) rather than
+// fetched from a table (random).
 // `id_add` (sharded build): the ids of this rank's slice start there; the slice itself is stored from 0.
+template <int MODE>
+__device__ __forceinline__ void assign_position(uint32_t p, uint32_t rank, uint32_t* __restrict__ tmp, const LevelTable& tab, void* __restrict__ uniq,
+                                                int S, const uint32_t* __restrict__ children, uint32_t n_children, uint32_t id_add = 0u) {
+  const uint32_t t = MODE == MODE_NODE ? 0u : tmp[p];
+  const uint32_t s = t & IDX_MASK;
+  uint32_t flags = t & ~IDX_MASK;
+  if (MODE == MODE_LEAF_DIRECT && (s & LEAF_SIDE)) {
+    reinterpret_cast<unsigned long long*>(uniq)[rank] = __ldcg(&tab.slots[s & (LEAF_SIDE - 1u)].key);
+    flags &= ~LEAF_SIDE;
+  } else if (MODE == MODE_LEAF_DIRECT) {
+    tab.dids[s] = rank;
+    reinterpret_cast<unsigned long long*>(uniq)[rank] = leaf_from_2bit(s, S);
+  } else if (MODE == MODE_LEAF_HASH) {
+    reinterpret_cast<unsigned long long*>(uniq)[rank] = (s == tab.cap) ? EMPTY_KEY : __ldcg(&tab.slots[s].key);
+  } else {
+    uint32_t l, r, cl, cr;
+    load_children(children, n_children, p, l, r);
+    canonical_node(l, r, cl, cr, flags);
+    reinterpret_cast<uint2*>(uniq)[rank] = make_uint2(cl, cr);
+  }
+  tmp[p] = finish_pointer(id_add + rank, flags);
+}
+
+// First occurrences of one tile: id = rank in position order.
 template <int MODE>
 __device__ __forceinline__ void assign_tile(uint32_t block, uint32_t base, const uint32_t (&words)[LVL_ITERS], const uint32_t* word_pref,
                                             uint32_t* __restrict__ tmp, uint32_t n, const LevelTable& tab, void* __restrict__ uniq, int S,
@@ -67,24 +91,7 @@ __device__ __forceinline__ void assign_tile(uint32_t block, uint32_t base, const
     const uint32_t p = block * LVL_TILE + it * LVL_THREADS + threadIdx.x;
     if (p < n && ((words[it] >> lane) & 1u)) {
       const uint32_t rank = base + word_pref[it * (LVL_THREADS / 32) + warp] + __popc(words[it] & ((1u << lane) - 1u));
-      const uint32_t t = MODE == MODE_NODE ? 0u : tmp[p];
-      const uint32_t s = t & IDX_MASK;
-      uint32_t flags = t & ~IDX_MASK;
-      if (MODE == MODE_LEAF_DIRECT && (s & LEAF_SIDE)) {
-        reinterpret_cast<unsigned long long*>(uniq)[rank] = __ldcg(&tab.slots[s & (LEAF_SIDE - 1u)].key);
-        flags &= ~LEAF_SIDE;
-      } else if (MODE == MODE_LEAF_DIRECT) {
-        tab.dids[s] = rank;
-        reinterpret_cast<unsigned long long*>(uniq)[rank] = leaf_from_2bit(s, S);
-      } else if (MODE == MODE_LEAF_HASH) {
-        reinterpret_cast<unsigned long long*>(uniq)[rank] = (s == tab.cap) ? EMPTY_KEY : __ldcg(&tab.slots[s].key);
-      } else {
-        uint32_t l, r, cl, cr;
-        load_children(children, n_children, p, l, r);
-        canonical_node(l, r, cl, cr, flags);
-        reinterpret_cast<uint2*>(uniq)[rank] = make_uint2(cl, cr);
-      }
-      tmp[p] = finish_pointer(id_add + rank, flags);
+      assign_position<MODE>(p, rank, tmp, tab, uniq, S, children, n_children, id_add);
     }
   }
 }
@@ -98,10 +105,20 @@ __device__ __forceinline__ void assign_tile(uint32_t block, uint32_t base, const
 // chains through every tile in flight and the kernel was 2-4x slower than this, profiles/README.md.)
 constexpr uint32_t CHUNK_TILES = 256;
 
+// `wpref` (optional, the rank directory below): receives the exclusive prefix of the popcounts of the
+// tile's 32 bitmap words, at the words' indices counted from the window's first tile.
 __device__ __forceinline__ void count_tile(const uint32_t* __restrict__ bitmask, uint32_t tile, uint32_t rel, uint32_t* __restrict__ blockcnt,
-                                           uint32_t* __restrict__ chunkcnt) {
+                                           uint32_t* __restrict__ chunkcnt, uint16_t* __restrict__ wpref = nullptr) {
   const uint32_t lane = threadIdx.x & 31;
-  const uint32_t c = warp_sum((uint32_t)__popc(bitmask[(uint64_t)tile * (LVL_TILE / 32) + lane]));
+  const uint32_t v = __popc(bitmask[(uint64_t)tile * (LVL_TILE / 32) + lane]);
+  uint32_t c;
+  if (wpref) {
+    const uint32_t x = warp_inclusive_sum(v);
+    wpref[(uint64_t)rel * (LVL_TILE / 32) + lane] = (uint16_t)(x - v);
+    c = __shfl_sync(0xffffffffu, x, 31);
+  } else {
+    c = warp_sum(v);
+  }
   if (lane == 0) {
     blockcnt[rel] = c;
     if (c) atomicAdd(chunkcnt + rel / CHUNK_TILES, c);
@@ -111,9 +128,36 @@ __device__ __forceinline__ void count_tile(const uint32_t* __restrict__ bitmask,
 // one warp per tile; tiles [first_block, first_block + nb) of the level, counts indexed from 0
 static __global__ void __launch_bounds__(256)
 count_kernel(const uint32_t* __restrict__ bitmask, uint32_t first_block, uint32_t nb, uint32_t* __restrict__ blockcnt,
-             uint32_t* __restrict__ chunkcnt) {
+             uint32_t* __restrict__ chunkcnt, uint16_t* __restrict__ wpref = nullptr) {
   const uint32_t rel = (blockIdx.x * 256 + threadIdx.x) >> 5;
-  if (rel < nb) count_tile(bitmask, first_block + rel, rel, blockcnt, chunkcnt);
+  if (rel < nb) count_tile(bitmask, first_block + rel, rel, blockcnt, chunkcnt, wpref);
+}
+
+// Rank directory of a whole level (node levels of the one-shot build, DESIGN.md §4).  Once the level's
+// bitmap is final, the id of any first occurrence q is
+//   tilebase[q / LVL_TILE] + wpref[q / 32] + popc(bitmap[q / 32] & lanes below q % 32),
+// so a later occurrence finds the id of its first occurrence without reading that position's pointer,
+// and both are finished in one pass.  Bitmap (n / 8 bytes), word prefixes (n / 16 bytes; a tile holds at
+// most 1024 first occurrences, 16 bits) and tile bases (n / 256 bytes) are all L2-sized.
+struct RankDir {
+  uint16_t* wpref;     // per bitmap word: first occurrences before it in its tile (count_kernel)
+  uint32_t* tilebase;  // per tile: first occurrences before it in the level (tile_bases_kernel)
+};
+
+// One CTA of CHUNK_TILES threads per chunk of tiles: tilebase[tile] = the chunk totals before the chunk
+// + the tile counts before the tile inside it.  The last CTA leaves the level's total in *total_out.
+static __global__ void __launch_bounds__(CHUNK_TILES)
+tile_bases_kernel(const uint32_t* __restrict__ blockcnt, const uint32_t* __restrict__ chunkcnt, uint32_t nb, uint32_t* __restrict__ tilebase,
+                  uint32_t* __restrict__ total_out) {
+  __shared__ uint32_t red_a[CHUNK_TILES / 32], red_b[CHUNK_TILES / 32];
+  const uint32_t chunk = blockIdx.x, tile = chunk * CHUNK_TILES + threadIdx.x;
+  uint32_t before = 0;
+  for (uint32_t i = threadIdx.x; i < chunk; i += CHUNK_TILES) before += chunkcnt[i];
+  uint32_t chunk_base, chunk_total;
+  block_exclusive_sum<CHUNK_TILES>(before, red_a, &chunk_base);
+  const uint32_t in_chunk = block_exclusive_sum<CHUNK_TILES>(tile < nb ? blockcnt[tile] : 0u, red_b, &chunk_total);
+  if (tile < nb) tilebase[tile] = chunk_base + in_chunk;
+  if (chunk == gridDim.x - 1 && threadIdx.x == 0) *total_out = chunk_base + chunk_total;
 }
 
 // Sum over the CTA of: the chunk totals before tile `rel`'s chunk + the tile counts before it in

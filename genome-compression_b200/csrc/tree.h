@@ -36,6 +36,8 @@ struct Options {
   uint64_t leaf_prefix_log2 = 25;        // one-shot ACGT-12 leaf level: after this many positions the ids seen so far are final and
                                          // the rest of the leaves look them up (build.cu: leaf_insert_acgt12_kernel); 0 = one window
   uint64_t profile_levels = 0;           // the kernel timings of stb_profile_read are kept per level ("name@L3")
+  uint64_t fused_resolve = 1;            // node levels of the one-shot build resolve their later occurrences in the assign pass,
+                                         // from a rank directory (build.cu: assign_resolve_kernel); 0 = separate resolve pass
 };
 
 struct Tree : Ctx {

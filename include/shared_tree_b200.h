@@ -66,7 +66,8 @@ int stb_release_workspace(stb_tree* tree);
 /* Tunables of the build (thresholds between its code paths; DESIGN.md §4).  Defaults are the
  * measured optimum; tests lower them to push small inputs through the large-input paths.
  * Names: "bucket_min", "bucket_levels", "bucket_cap", "partition_threads", "dedup_threads", "bucket_slack_permille", "bucket_headroom", "child_filter", "locality",
- * "coop_max", "reserve_pipeline", "side_table_slots", "stream_chunk_log2", "stream_min_chunks", "leaf_prefix_log2", "profile_levels".  Unknown name: STB_ERR_INVALID_ARG. */
+ * "coop_max", "reserve_pipeline", "side_table_slots", "stream_chunk_log2", "stream_min_chunks", "leaf_prefix_log2", "profile_levels",
+ * "fused_resolve".  Unknown name: STB_ERR_INVALID_ARG. */
 int stb_set_option(stb_tree* tree, const char* name, uint64_t value);
 int stb_get_option(const stb_tree* tree, const char* name, uint64_t* value);
 
@@ -144,6 +145,8 @@ int stb_profile_enable(stb_tree* tree, int on);
 int stb_profile_reset(stb_tree* tree);
 /* Fills names[i] (static strings), total_ms[i], launches[i] for up to cap kernel
  * classes; *count receives the number of classes.
+ * A level's ids: count_firsts, then assign_ids and resolve_ids; node levels built one kernel at a time
+ * with the option fused_resolve (default) run tile_bases and assign_resolve instead of the last two.
  * Besides the kernels, five classes with total_ms = 0 count the on-chip (bucketed) node levels of the
  * builds profiled, one per level, by what that level's deduplication came to:
  *   dedup_on_chip              every final bucket fitted its region
