@@ -85,6 +85,7 @@ def _load() -> C.CDLL:
         "stb_decode_leaves": [vp, u64, u64, vp, i32],
         "stb_decode_ascii": [vp, u64, u64, vp, i32],
         "stb_random_access": [vp, vp, u64, vp, i32],
+        "stb_extract_regions": [vp, vp, vp, vp, u64, vp, u64, i32, P(u64)],
         "stb_profile_enable": [vp, i32],
         "stb_profile_reset": [vp],
         "stb_profile_read": [vp, P(cp), P(C.c_double), P(u64), u64, P(u64)],
@@ -333,6 +334,35 @@ class SharedTree:
         res = np.zeros(idx.size, dtype=np.uint64)
         self._check(lib.stb_random_access(self._h, idx.ctypes.data, idx.size, res.ctypes.data, HOST))
         return res
+
+    def extract_regions(self, start, end, strand=None, out=None):
+        """Bases [start[i], end[i]) of the sequence (0-based, half-open as in BED), strand[i] = 1 for the reverse
+        complement, back to back in input order (stb_extract_regions).  Host arrays: returns the letters as bytes.
+        CUDA tensors (8-byte start / end, uint8 strand and out): fills out and returns the total length; without
+        out, only returns the total length."""
+        if _is_device_tensor(start):
+            for x, size in ((start, 8), (end, 8), (strand, 1), (out, 1)):
+                if x is not None:
+                    assert _is_device_tensor(x) and x.is_contiguous() and x.element_size() == size, \
+                        "device regions: contiguous CUDA tensors, 8-byte start / end, uint8 strand and out"
+            assert end.numel() == start.numel() and (strand is None or strand.numel() == start.numel())
+            written = C.c_uint64(0)
+            self._check(lib.stb_extract_regions(self._h, start.data_ptr(), end.data_ptr(),
+                                                None if strand is None else strand.data_ptr(), start.numel(),
+                                                None if out is None else out.data_ptr(), 0 if out is None else out.numel(),
+                                                DEVICE, C.byref(written)))
+            return int(written.value)
+        s = np.ascontiguousarray(start, dtype=np.uint64)
+        e = np.ascontiguousarray(end, dtype=np.uint64)
+        st = None if strand is None else np.ascontiguousarray(strand, dtype=np.uint8)
+        assert e.size == s.size and (st is None or st.size == s.size)
+        # sized here when the regions are ordered; otherwise the call reports them before writing anything
+        total = int((e - s).sum(dtype=np.uint64)) if bool((e >= s).all()) else 0
+        res = np.zeros(max(total, 1), dtype=np.uint8)
+        written = C.c_uint64(0)
+        self._check(lib.stb_extract_regions(self._h, s.ctypes.data, e.ctypes.data, None if st is None else st.ctypes.data,
+                                            s.size, res.ctypes.data, total, HOST, C.byref(written)))
+        return res[:written.value].tobytes()
 
     def __getitem__(self, i: int) -> int:
         return int(self.random_access(np.array([i], dtype=np.uint64))[0])

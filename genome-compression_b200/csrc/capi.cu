@@ -500,6 +500,47 @@ int stb_random_access(const stb_tree* tree, const uint64_t* index, uint64_t quer
   return from_device(t, reinterpret_cast<unsigned long long*>(out), d_out.ptr, queries, STB_HOST);
 }
 
+int stb_extract_regions(const stb_tree* tree, const uint64_t* start, const uint64_t* end, const uint8_t* strand,
+                        uint64_t n_regions, char* out, uint64_t cap, int memory, uint64_t* written) {
+  if (!tree || !written || !valid_memory(memory)) return STB_ERR_INVALID_ARG;
+  if (!tree->built) return tree->fail(STB_ERR_NOT_BUILT, "tree is empty");
+  if (n_regions == 0) {
+    *written = 0;
+    return STB_OK;
+  }
+  if (!start || !end) return tree->fail(STB_ERR_INVALID_ARG, "extract_regions: null start or end array");
+  STB_TRY(use_device(tree));
+  Tree& t = const_cast<stb_tree&>(*tree);
+  auto d_start = reinterpret_cast<const unsigned long long*>(start), d_end = reinterpret_cast<const unsigned long long*>(end);
+  const uint8_t* d_strand = strand;
+  if (memory == STB_DEVICE) {
+    if ((reinterpret_cast<uintptr_t>(start) | reinterpret_cast<uintptr_t>(end)) & 7u)
+      return t.fail(STB_ERR_INVALID_ARG, "extract_regions: start and end must be 8-byte aligned");
+  } else {
+    const uint64_t words = 8 * n_regions;
+    STB_CUDA(t, t.region_inputs.ensure(2 * words + (strand ? n_regions : 0), t.stream));
+    char* d = t.region_inputs.ptr;
+    Launch l(t, "h2d_copy", false);
+    STB_CUDA(t, cudaMemcpyAsync(d, start, words, cudaMemcpyHostToDevice, t.stream));
+    STB_CUDA(t, cudaMemcpyAsync(d + words, end, words, cudaMemcpyHostToDevice, t.stream));
+    if (strand) STB_CUDA(t, cudaMemcpyAsync(d + 2 * words, strand, n_regions, cudaMemcpyHostToDevice, t.stream));
+    d_start = reinterpret_cast<const unsigned long long*>(d);
+    d_end = reinterpret_cast<const unsigned long long*>(d + words);
+    d_strand = strand ? reinterpret_cast<const uint8_t*>(d + 2 * words) : nullptr;
+  }
+  RegionPlan plan;
+  STB_TRY(region_plan(t, d_start, d_end, d_strand, n_regions, &plan));
+  const uint64_t total = plan.total_len;
+  *written = total;
+  if (!out) return STB_OK;
+  if (cap < total) return t.fail(STB_ERR_BUFFER_TOO_SMALL, "extract_regions: cap < total region length");
+  if (memory == STB_DEVICE) return region_write(t, d_start, d_end, d_strand, n_regions, plan, out);
+  // the output comes back through the handle's grow-only staging buffer
+  STB_CUDA(t, t.staging.ensure(total + 16, t.stream));
+  STB_TRY(region_write(t, d_start, d_end, d_strand, n_regions, plan, t.staging.ptr));
+  return from_device(t, out, t.staging.ptr, total, STB_HOST);
+}
+
 const char* stb_status_string(int status) {
   switch (status) {
     case STB_OK: return "ok";

@@ -9,6 +9,7 @@
 // requested leaf range, so decoding `count` leaves costs O(count + depth).
 #include <algorithm>
 
+#include "scan.cuh"
 #include "staging.cuh"
 #include "tree.h"
 
@@ -248,21 +249,12 @@ fused_ascii_kernel(const uint32_t* __restrict__ cur, unsigned long long lo_cur, 
   copy_out_staged<FA_THREADS>(out + dst - shift, stage, shift, (uint32_t)(tile_hi - tile_lo) * S);
 }
 
-// operator[] batched: one thread per query, depth dependent gathers.
-__global__ void __launch_bounds__(DEC_THREADS)
-random_access_kernel(const unsigned long long* __restrict__ index, unsigned long long q, LayerPtrs layers, int n_layers,
-                     uint32_t root, const unsigned long long* __restrict__ leaves, int S, unsigned long long width,
-                     unsigned long long* __restrict__ out, uint32_t* __restrict__ out_of_range) {
-  const unsigned long long j = (unsigned long long)blockIdx.x * DEC_THREADS + threadIdx.x;
-  if (j >= q) return;
-  unsigned long long idx = index[j];
-  if (idx >= width) {
-    *out_of_range = 1u;
-    out[j] = 0ull;
-    return;
-  }
+// operator[]'s descent (:268-291) from the root through node layers n_layers-1 .. stop: returns the pointer
+// into node layer stop-1 (stop = 0: the leaf pointer) on the path to leaf `idx` (< width()).
+__device__ __forceinline__ uint32_t descend(const LayerPtrs& layers, int n_layers, uint32_t root, unsigned long long idx,
+                                            int stop) {
   uint32_t cur = root;
-  for (int layer = n_layers - 1; layer >= 0; --layer) {
+  for (int layer = n_layers - 1; layer >= stop; --layer) {
     const uint2 nd = __ldg(layers.nodes[layer] + (cur & IDX_MASK));
     const uint32_t m = (cur >> 29) & 1u, t = (cur >> 30) & 1u;
     const unsigned long long size = 1ull << layer;  // leaves under the logical left child (:272)
@@ -274,7 +266,183 @@ random_access_kernel(const unsigned long long* __restrict__ index, unsigned long
     const uint32_t child = (side ^ m) ? nd.y : nd.x;
     cur = compose(child, m, t);
   }
+  return cur;
+}
+
+// operator[] batched: one thread per query, depth dependent gathers.
+__global__ void __launch_bounds__(DEC_THREADS)
+random_access_kernel(const unsigned long long* __restrict__ index, unsigned long long q, LayerPtrs layers, int n_layers,
+                     uint32_t root, const unsigned long long* __restrict__ leaves, int S, unsigned long long width,
+                     unsigned long long* __restrict__ out, uint32_t* __restrict__ out_of_range) {
+  const unsigned long long j = (unsigned long long)blockIdx.x * DEC_THREADS + threadIdx.x;
+  if (j >= q) return;
+  const unsigned long long idx = index[j];
+  if (idx >= width) {
+    *out_of_range = 1u;
+    out[j] = 0ull;
+    return;
+  }
+  const uint32_t cur = descend(layers, n_layers, root, idx, 0);
   out[j] = apply_leaf(__ldg(leaves + (cur & IDX_MASK)), cur, S);
+}
+
+// ---- region extraction ------------------------------------------------------------------------
+// A work item is one (region, aligned group of FUSE_LEAVES leaves the region touches).  A region's items are
+// numbered in output order: first group to last on strand 0, last group to first on strand 1, so the items
+// [t0, t1) of a CTA write one contiguous byte range.  Scratch per region: item base and output offset
+// (exclusive scans of the item counts and of the lengths; RC_THREADS-region blocks first, then the block
+// totals, then the sum of the two).
+constexpr int RC_THREADS = 1024;
+constexpr int RX_THREADS = 128;
+// bits of the flag word the count kernel raises
+constexpr unsigned long long REGION_BAD_ORDER = 1, REGION_BAD_END = 2, REGION_BAD_STRAND = 4;
+// Regions of at least this many bases take their groups' pointers from one level expansion (expand_levels) over
+// the hull of all such regions of the call instead of descending from the root per group.  One expansion costs a
+// fixed chain of about 25 launches, which only regions this long repay; on the config-3 tree it takes the
+// whole sequence as 24 regions from 4.66 to 4.60 ms (DESIGN.md, profiles/r05_regions_3100mbp*.json).
+constexpr unsigned long long REGION_EXPAND_MIN = 1ull << 25;
+
+__global__ void __launch_bounds__(RC_THREADS)
+region_count_kernel(const unsigned long long* __restrict__ start, const unsigned long long* __restrict__ end,
+                    const uint8_t* __restrict__ strand, unsigned long long n, unsigned long long limit, int S,
+                    unsigned long long long_min, unsigned long long* __restrict__ item_base,
+                    unsigned long long* __restrict__ out_off, unsigned long long* __restrict__ block_items,
+                    unsigned long long* __restrict__ block_len, unsigned long long* __restrict__ flags) {
+  __shared__ unsigned long long warp_totals[RC_THREADS / 32];
+  const unsigned long long i = (unsigned long long)blockIdx.x * RC_THREADS + threadIdx.x;
+  unsigned long long len = 0, items = 0;
+  if (i < n) {
+    const unsigned long long s = start[i], e = end[i];
+    unsigned long long bad = 0;
+    if (s > e) bad |= REGION_BAD_ORDER;
+    if (e > limit) bad |= REGION_BAD_END;
+    if (strand && strand[i] > 1) bad |= REGION_BAD_STRAND;
+    if (bad) {
+      atomicOr(flags, bad);
+    } else if (e > s) {
+      len = e - s;
+      const unsigned long long g0 = (s / (unsigned)S) >> FUSE, g1 = ((e - 1) / (unsigned)S) >> FUSE;
+      items = g1 - g0 + 1;
+      if (len >= long_min) {  // flags[1] = last group of the hull, flags[2] = ~its first group (0: no hull)
+        atomicMax(flags + 1, g1);
+        atomicMax(flags + 2, ~g0);
+      }
+    }
+  }
+  unsigned long long total;
+  const unsigned long long ib = block_exclusive_sum<RC_THREADS>(items, warp_totals, &total);
+  if (i < n) item_base[i] = ib;
+  if (threadIdx.x == 0) block_items[blockIdx.x] = total;
+  __syncthreads();  // warp_totals is written again
+  const unsigned long long ob = block_exclusive_sum<RC_THREADS>(len, warp_totals, &total);
+  if (i < n) out_off[i] = ob;
+  if (threadIdx.x == 0) block_len[blockIdx.x] = total;
+}
+
+// One CTA: the block totals become block bases; summary[0] = total length, summary[1] = total items.
+__global__ void __launch_bounds__(1024)
+region_scan_kernel(unsigned long long* __restrict__ block_items, unsigned long long* __restrict__ block_len, uint32_t blocks,
+                   unsigned long long* __restrict__ summary) {
+  const unsigned long long items = cta_exclusive_scan(block_items, block_items, blocks);
+  const unsigned long long len = cta_exclusive_scan(block_len, block_len, blocks);
+  if (threadIdx.x == 0) {
+    summary[0] = len;
+    summary[1] = items;
+  }
+}
+
+__global__ void __launch_bounds__(RC_THREADS)
+region_base_kernel(unsigned long long* __restrict__ item_base, unsigned long long* __restrict__ out_off,
+                   const unsigned long long* __restrict__ block_items, const unsigned long long* __restrict__ block_len,
+                   unsigned long long n) {
+  const unsigned long long i = (unsigned long long)blockIdx.x * RC_THREADS + threadIdx.x;
+  if (i >= n) return;
+  item_base[i] += block_items[blockIdx.x];
+  out_off[i] += block_len[blockIdx.x];
+}
+
+// Thread = item: finds its region (the last one whose item base is <= the item), takes the group's pointer
+// into node layer FUSE-1 from the hull's expansion (regions of at least long_min bases) or on operator[]'s path
+// (or, in trees of fewer than FUSE node layers, each leaf's pointer),
+// walks the group, and spells the bases inside the region into the CTA's staged range, strand 1 through
+// leaf_inverted and in reverse order.  The range leaves the SM as aligned words.
+__global__ void __launch_bounds__(RX_THREADS)
+extract_regions_kernel(const unsigned long long* __restrict__ start, const unsigned long long* __restrict__ end,
+                       const uint8_t* __restrict__ strand, const unsigned long long* __restrict__ item_base,
+                       const unsigned long long* __restrict__ out_off, unsigned long long n_regions, unsigned long long n_items,
+                       LayerPtrs layers, int n_layers, uint32_t root, const unsigned long long* __restrict__ leaves, int S,
+                       unsigned long long width, const uint32_t* __restrict__ hull, unsigned long long hull_lo,
+                       unsigned long long long_min, char* __restrict__ out) {
+  __shared__ __align__(16) uint8_t stage[RX_THREADS * FUSE_LEAVES * 16 + 16];
+  __shared__ unsigned long long range[2];  // the CTA's output bytes [range[0], range[1])
+  const unsigned long long item = (unsigned long long)blockIdx.x * RX_THREADS + threadIdx.x;
+  const bool active = item < n_items;
+  unsigned long long lo = 0, hi = 0, o_start = 0, g = 0;
+  bool rev = false;
+  unsigned long long v[FUSE_LEAVES];
+#pragma unroll
+  for (int i = 0; i < FUSE_LEAVES; ++i) v[i] = 0ull;
+  if (active) {
+    unsigned long long a = 0, b = n_regions;  // item_base[a] <= item < item_base[b] (item_base[n_regions] = n_items)
+    while (b - a > 1) {
+      const unsigned long long mid = a + (b - a) / 2;
+      if (item_base[mid] <= item) a = mid;
+      else b = mid;
+    }
+    const unsigned long long s = start[a], e = end[a];
+    rev = strand && strand[a];
+    const unsigned long long span = (unsigned long long)S * FUSE_LEAVES;  // bases of a group
+    const unsigned long long j = item - item_base[a];
+    g = rev ? ((e - 1) / (unsigned)S >> FUSE) - j : (s / (unsigned)S >> FUSE) + j;
+    lo = max(s, g * span);
+    hi = min(e, g * span + span);
+    o_start = out_off[a] + (rev ? e - hi : lo - s);
+    if (threadIdx.x == 0) range[0] = o_start;
+    if (item + 1 == n_items || threadIdx.x == RX_THREADS - 1) range[1] = o_start + (hi - lo);
+    const unsigned long long first_leaf = g * FUSE_LEAVES;
+    auto wanted = [&](uint32_t slot) {  // does leaf `slot` of the group hold a base of [lo, hi)?
+      const unsigned long long b0 = (first_leaf + slot) * (unsigned)S;
+      return b0 < hi && b0 + (unsigned)S > lo;
+    };
+    if (n_layers >= FUSE) {
+      const uint32_t p2 = e - s >= long_min ? hull[g - hull_lo] : descend(layers, n_layers, root, first_leaf, FUSE);
+      walk_subtree(p2, layers.nodes[2], layers.nodes[1], layers.nodes[0],
+                   [&](uint32_t slot, uint32_t lp) {
+                     if (!wanted(slot)) return;
+                     const unsigned long long x = apply_leaf(__ldg(leaves + (lp & IDX_MASK)), lp, S);
+#pragma unroll
+                     for (int i = 0; i < FUSE_LEAVES; ++i)
+                       if (slot == (uint32_t)i) v[i] = x;
+                   });
+    } else {  // at most 2^n_layers < FUSE_LEAVES leaves, all in group 0
+#pragma unroll
+      for (int i = 0; i < FUSE_LEAVES; ++i)
+        if (i < width && wanted(i)) {
+          const uint32_t lp = descend(layers, n_layers, root, i, 0);
+          v[i] = apply_leaf(__ldg(leaves + (lp & IDX_MASK)), lp, S);
+        }
+    }
+  }
+  __syncthreads();
+  const unsigned long long base = range[0];
+  const uint32_t shift = (uint32_t)((reinterpret_cast<uintptr_t>(out) + base) & 3ull);
+  if (active) {
+#pragma unroll
+    for (int i = 0; i < FUSE_LEAVES; ++i) {
+      const unsigned long long b0 = (g * FUSE_LEAVES + i) * (unsigned)S;  // first base of the leaf
+      const unsigned long long a = max(lo, b0), b = min(hi, b0 + (unsigned)S);
+      if (a >= b) continue;
+      if (rev) {  // leaf_inverted's letter k is the complement of base b0 + S-1-k
+        const uint32_t at = shift + (uint32_t)(o_start + (hi - b) - base);
+        spell_bytes(stage + at, leaf_inverted(v[i], S) >> (4 * (b0 + S - b)), (int)(b - a));
+      } else {
+        const uint32_t at = shift + (uint32_t)(o_start + (a - lo) - base);
+        spell_bytes(stage + at, v[i] >> (4 * (a - b0)), (int)(b - a));
+      }
+    }
+  }
+  __syncthreads();
+  copy_out_staged<RX_THREADS>(out + base - shift, stage, shift, (uint32_t)(range[1] - base));
 }
 
 // width() for a tree that was not built here: nulls exist only on the logical right
@@ -335,17 +503,13 @@ int decode_reserve(Tree& t) {
   return STB_OK;
 }
 
-int decode_range(const Tree& tc, uint64_t first, uint64_t count, unsigned long long* d_out, char* d_ascii) {
-  Tree& t = const_cast<Tree&>(tc);
-  if (!t.built) return t.fail(STB_ERR_NOT_BUILT, "tree is empty");
-  if (count == 0) return STB_OK;
-  if (first + count > t.width || first + count < first) return t.fail(STB_ERR_OUT_OF_RANGE, "decode range exceeds width()");
+// The top-down expansion over leaves [first, last] down to pointer level stop-1 (pointer level k refers to node
+// layer k and covers 2^(k+1) leaves; level -1 = leaf pointers): *cur receives that level's array (t.decode_a or
+// t.decode_b), whose entry 0 is position *lo_cur.  Enqueued only: the caller synchronises before t.root may change.
+static int expand_levels(Tree& t, uint64_t first, uint64_t last, int stop, uint32_t** cur_out, uint64_t* lo_out) {
   cudaStream_t st = t.stream;
   const int L = (int)t.layers.size();
-  const uint64_t last = first + count - 1;
-  // pointer level k refers to node layer k and covers 2^(k+1) leaves; level -1 = leaf pointers
-  const int stop = L >= FUSE ? FUSE : 0;  // pointer levels below `stop` are walked inside the output kernel
-  // the largest pointer array that is ever materialised: the one entering the output kernel
+  // the largest pointer array that is ever materialised: the last one
   const uint64_t widest = ((last >> stop) - (first >> stop) + 1) * (stop ? 1 : 2) + 2;
   STB_CUDA(t, t.decode_a.ensure(widest, st));
   STB_CUDA(t, t.decode_b.ensure(widest, st));
@@ -363,6 +527,23 @@ int decode_range(const Tree& tc, uint64_t first, uint64_t count, unsigned long l
     std::swap(cur, nxt);
     lo_cur = lo_next;
   }
+  *cur_out = cur;
+  *lo_out = lo_cur;
+  return STB_OK;
+}
+
+int decode_range(const Tree& tc, uint64_t first, uint64_t count, unsigned long long* d_out, char* d_ascii) {
+  Tree& t = const_cast<Tree&>(tc);
+  if (!t.built) return t.fail(STB_ERR_NOT_BUILT, "tree is empty");
+  if (count == 0) return STB_OK;
+  if (first + count > t.width || first + count < first) return t.fail(STB_ERR_OUT_OF_RANGE, "decode range exceeds width()");
+  cudaStream_t st = t.stream;
+  const int L = (int)t.layers.size();
+  const uint64_t last = first + count - 1;
+  const int stop = L >= FUSE ? FUSE : 0;  // pointer levels below `stop` are walked inside the output kernel
+  uint32_t* cur = nullptr;
+  uint64_t lo_cur = 0;
+  STB_TRY(expand_levels(t, first, last, stop, &cur, &lo_cur));
   if (stop) {
     const uint2 *l2 = t.layers[2].nodes.ptr, *l1 = t.layers[1].nodes.ptr, *l0 = t.layers[0].nodes.ptr;
     if (d_out) {
@@ -440,6 +621,76 @@ int random_access(const Tree& tc, const unsigned long long* d_index, uint64_t q,
   STB_CUDA(t, cudaStreamSynchronize(t.stream));
   STB_CUDA(t, cudaGetLastError());
   if (h) return t.fail(STB_ERR_OUT_OF_RANGE, "random access index >= width()");
+  return STB_OK;
+}
+
+// t.region_scratch: item bases [n], output offsets [n], block bases of each [blocks], summary [5]: total length,
+// total items, error flags, hull of the long regions (last group, ~first group)
+static uint64_t region_blocks(uint64_t n) { return ceil_div(n, RC_THREADS); }
+
+int region_plan(const Tree& tc, const unsigned long long* d_start, const unsigned long long* d_end, const uint8_t* d_strand,
+                uint64_t n, RegionPlan* plan) {
+  Tree& t = const_cast<Tree&>(tc);
+  if (!t.built) return t.fail(STB_ERR_NOT_BUILT, "tree is empty");
+  cudaStream_t st = t.stream;
+  const uint64_t blocks = region_blocks(n);
+  STB_CUDA(t, t.region_scratch.ensure(2 * n + 2 * blocks + 5, st));
+  unsigned long long* item_base = t.region_scratch.ptr;
+  unsigned long long* out_off = item_base + n;
+  unsigned long long* block_items = out_off + n;
+  unsigned long long* block_len = block_items + blocks;
+  unsigned long long* summary = block_len + blocks;
+  STB_CUDA(t, cudaMemsetAsync(summary + 2, 0, 3 * 8, st));
+  const unsigned long long long_min = t.layers.size() >= FUSE ? REGION_EXPAND_MIN : ~0ull;
+  {
+    Launch l(t, "region_count");
+    region_count_kernel<<<(unsigned)blocks, RC_THREADS, 0, st>>>(d_start, d_end, d_strand, n, t.width * (uint64_t)t.S, t.S,
+                                                                 long_min, item_base, out_off, block_items, block_len,
+                                                                 summary + 2);
+  }
+  {
+    Launch l(t, "region_scan");
+    region_scan_kernel<<<1, 1024, 0, st>>>(block_items, block_len, (uint32_t)blocks, summary);
+  }
+  {
+    Launch l(t, "region_base");
+    region_base_kernel<<<(unsigned)blocks, RC_THREADS, 0, st>>>(item_base, out_off, block_items, block_len, n);
+  }
+  unsigned long long h[5] = {0, 0, 0, 0, 0};
+  STB_CUDA(t, cudaMemcpyAsync(h, summary, sizeof(h), cudaMemcpyDeviceToHost, st));
+  STB_CUDA(t, cudaStreamSynchronize(st));
+  STB_CUDA(t, cudaGetLastError());
+  if (h[2] & REGION_BAD_ORDER) return t.fail(STB_ERR_INVALID_ARG, "region start > end");
+  if (h[2] & REGION_BAD_STRAND) return t.fail(STB_ERR_INVALID_ARG, "region strand is neither 0 nor 1");
+  if (h[2] & REGION_BAD_END) return t.fail(STB_ERR_OUT_OF_RANGE, "region end > width() * dna_size");
+  plan->total_len = h[0];
+  plan->items = h[1];
+  plan->hull = h[4] != 0;
+  plan->hull_first = ~h[4];
+  plan->hull_last = h[3];
+  return STB_OK;
+}
+
+int region_write(const Tree& tc, const unsigned long long* d_start, const unsigned long long* d_end, const uint8_t* d_strand,
+                 uint64_t n, const RegionPlan& plan, char* d_out) {
+  Tree& t = const_cast<Tree&>(tc);
+  if (plan.items == 0) return STB_OK;
+  LayerPtrs lp{};
+  STB_TRY(layer_ptrs(t, lp));
+  const unsigned long long* item_base = t.region_scratch.ptr;
+  uint32_t* hull = nullptr;
+  uint64_t hull_lo = 0;
+  if (plan.hull)
+    STB_TRY(expand_levels(t, plan.hull_first << FUSE, std::min(t.width - 1, (plan.hull_last << FUSE) + FUSE_LEAVES - 1), FUSE,
+                          &hull, &hull_lo));
+  {
+    Launch l(t, "extract_regions");
+    extract_regions_kernel<<<(unsigned)ceil_div(plan.items, RX_THREADS), RX_THREADS, 0, t.stream>>>(
+        d_start, d_end, d_strand, item_base, item_base + n, n, plan.items, lp, (int)t.layers.size(), t.root, t.leaves.ptr,
+        t.S, t.width, hull, hull_lo, plan.hull ? REGION_EXPAND_MIN : ~0ull, d_out);
+  }
+  STB_CUDA(t, cudaStreamSynchronize(t.stream));
+  STB_CUDA(t, cudaGetLastError());
   return STB_OK;
 }
 

@@ -62,9 +62,15 @@ struct Tree : Ctx {
   // the handle has sorted a tree of this shape)
   DevBuf<unsigned long long> spare_leaves;
   std::vector<DevBuf<uint2>> spare_nodes;
+  // Scratch of region extraction: per-region item bases and output offsets (decode.cu: region_plan), and the
+  // region arrays of a host-memory call (t.staging carries that call's output back, so they cannot share it).
+  DevBuf<unsigned long long> region_scratch;
+  DevBuf<char> region_inputs;
   void release_scratch() {
     decode_a.release();
     decode_b.release();
+    region_scratch.release();
+    region_inputs.release();
     sort_arena.release();
     spare_leaves.release();
     spare_nodes.clear();
@@ -134,6 +140,17 @@ int compute_width(Tree& t);
 int decode_reserve(Tree& t);  // the scratch a full decode of this tree will need (kept by the handle)
 int decode_range(const Tree& t, uint64_t first, uint64_t count, unsigned long long* d_out, char* d_ascii);
 int random_access(const Tree& t, const unsigned long long* d_index, uint64_t q, unsigned long long* d_out);
+// stb_extract_regions in two steps on device arrays: region_plan checks every region and sizes the output
+// (the scratch it leaves on the handle is what region_write reads); region_write writes it.
+struct RegionPlan {
+  uint64_t total_len = 0, items = 0;
+  bool hull = false;  // some regions are long enough to be read from one level expansion over groups [hull_first, hull_last]
+  uint64_t hull_first = 0, hull_last = 0;
+};
+int region_plan(const Tree& t, const unsigned long long* d_start, const unsigned long long* d_end, const uint8_t* d_strand,
+                uint64_t n, RegionPlan* plan);
+int region_write(const Tree& t, const unsigned long long* d_start, const unsigned long long* d_end, const uint8_t* d_strand,
+                 uint64_t n, const RegionPlan& plan, char* d_out);
 
 // synth.cu -------------------------------------------------------------------------
 int synth_genome(Ctx& ctx, char* d_out, uint64_t n_bases, uint64_t first, uint64_t count, uint64_t seed,

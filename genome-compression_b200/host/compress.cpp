@@ -11,7 +11,9 @@
 #include <filesystem>
 #include <fstream>
 #include <iostream>
+#include <sstream>
 #include <string>
+#include <vector>
 
 #include "shared_tree.h"
 
@@ -19,7 +21,7 @@ namespace fs = std::filesystem;
 using clk = std::chrono::steady_clock;
 
 struct Options {
-  fs::path input, output, histogram;
+  fs::path input, output, histogram, regions;
   bool verbose = false, statistics = false, save = true, decompress = false;
   std::size_t dna_size = 12;
 };
@@ -33,7 +35,10 @@ static void usage() {
                "  --output=<file>      output path (default <input>.dag, or <input>.txt with --decompress)\n"
                "  --histogram=<file>   write per-layer reference-count histograms (CSV)\n"
                "  --dna-size=<n>       nucleotides per leaf, 1..16 (default 12)\n"
-               "  --decompress         input is a .dag file; write the decoded sequence as text\n";
+               "  --decompress         input is a .dag file; write the decoded sequence as text\n"
+               "  --regions=<file>     with --decompress: write only the regions of a BED file (chrom start end\n"
+               "                       [name [score [strand]]], 0-based half-open; strand '-' = reverse complement)\n"
+               "                       as FASTA, one record per region in file order (default output <input>.fa)\n";
 }
 
 static Options parse(int argc, char** argv) {
@@ -48,6 +53,7 @@ static Options parse(int argc, char** argv) {
     else if (a == "--decompress") o.decompress = true;
     else if (a.rfind("--output=", 0) == 0) o.output = value("--output=");
     else if (a.rfind("--histogram=", 0) == 0) o.histogram = value("--histogram=");
+    else if (a.rfind("--regions=", 0) == 0) o.regions = value("--regions=");
     else if (a.rfind("--dna-size=", 0) == 0) o.dna_size = (std::size_t)std::atoi(value("--dna-size=").c_str());
     else if (o.input.empty()) o.input = a;
     else { std::cout << "Compression of multiple files at once is currently not supported.\n"; std::exit(1); }
@@ -56,13 +62,99 @@ static Options parse(int argc, char** argv) {
   if (o.input.empty()) { std::cout << "Invalid command: argument <file> required.\nUse --help for more information\n"; std::exit(2); }
   if (o.dna_size < 1 || o.dna_size > 16) { std::cout << "Invalid --dna-size: 1..16 supported\n"; std::exit(2); }
   if (!fs::is_regular_file(o.input)) { std::cout << "Invalid filename: " << o.input << '\n'; std::exit(2); }
-  if (o.output.empty() && o.save) { o.output = o.input; o.output.replace_extension(o.decompress ? ".txt" : ".dag"); }
+  if (!o.regions.empty() && !o.decompress) { std::cout << "Invalid flag combination: --regions needs --decompress\n"; std::exit(2); }
+  if (o.output.empty() && o.save) {
+    o.output = o.input;
+    o.output.replace_extension(!o.decompress ? ".dag" : o.regions.empty() ? ".txt" : ".fa");
+  }
   return o;
 }
 
 static double ms_since(clk::time_point t0) { return std::chrono::duration<double, std::milli>(clk::now() - t0).count(); }
 
+struct Region {
+  std::string chrom;
+  uint64_t start = 0, end = 0;
+  uint8_t strand = 0;
+  std::size_t line = 0;
+};
+
+static bool parse_u64(const std::string& s, uint64_t& v) {
+  if (s.empty() || s.size() > 19 || s.find_first_not_of("0123456789") != std::string::npos) return false;
+  v = std::stoull(s);
+  return true;
+}
+
+[[noreturn]] static void bed_error(std::size_t line, const std::string& what) {
+  std::cerr << "line " << line << ": " << what << '\n';
+  std::exit(1);
+}
+
+// BED: whitespace-separated `chrom start end [name [score [strand]]]`; empty lines and lines starting with
+// '#', "track" or "browser" are skipped.  Any malformed line ends the program before the device is touched.
+static std::vector<Region> read_bed(const fs::path& path) {
+  std::ifstream in{path};
+  if (!in) { std::cerr << "cannot read " << path << '\n'; std::exit(1); }
+  std::vector<Region> regions;
+  std::string text;
+  for (std::size_t line = 1; std::getline(in, text); ++line) {
+    std::istringstream fields{text};
+    std::vector<std::string> f;
+    for (std::string w; fields >> w;) f.push_back(w);
+    if (f.empty() || f[0][0] == '#' || f[0] == "track" || f[0] == "browser") continue;
+    if (f.size() < 3) bed_error(line, "expected chrom, start and end");
+    Region r;
+    r.chrom = f[0];
+    r.line = line;
+    if (!parse_u64(f[1], r.start)) bed_error(line, "start is not a non-negative integer: " + f[1]);
+    if (!parse_u64(f[2], r.end)) bed_error(line, "end is not a non-negative integer: " + f[2]);
+    if (r.start > r.end) bed_error(line, "start " + f[1] + " > end " + f[2]);
+    if (f.size() >= 6) {
+      if (f[5] == "-") r.strand = 1;
+      else if (f[5] != "+" && f[5] != ".") bed_error(line, "strand is not '+', '-' or '.': " + f[5]);
+    }
+    regions.push_back(r);
+  }
+  return regions;
+}
+
+// One stb_extract_regions call for every region of the BED file, written as FASTA records.
+static int extract(const Options& o) {
+  const std::vector<Region> regions = read_bed(o.regions);
+  std::ifstream in{o.input, std::ios::binary};
+  shared_tree tree = shared_tree::deserialize(in);
+  const uint64_t bases = (uint64_t)tree.width() * dna::size();
+  std::vector<uint64_t> start(regions.size()), end(regions.size());
+  std::vector<uint8_t> strand(regions.size());
+  uint64_t total = 0;
+  for (std::size_t i = 0; i < regions.size(); ++i) {
+    const Region& r = regions[i];
+    if (r.end > bases) bed_error(r.line, "end " + std::to_string(r.end) + " is past the sequence (" + std::to_string(bases) + " bases)");
+    start[i] = r.start;
+    end[i] = r.end;
+    strand[i] = r.strand;
+    total += r.end - r.start;
+  }
+  std::string seq(total, '\0');
+  uint64_t written = 0;
+  const int st = stb_extract_regions(tree.handle(), start.data(), end.data(), strand.data(), regions.size(), seq.data(),
+                                     seq.size(), STB_HOST, &written);
+  if (st != STB_OK) { std::cerr << stb_last_error(tree.handle()) << '\n'; return 1; }
+  if (o.save) {
+    std::ofstream out{o.output, std::ios::binary};
+    uint64_t at = 0;
+    for (const Region& r : regions) {
+      out << '>' << r.chrom << ':' << r.start << '-' << r.end << '(' << (r.strand ? '-' : '+') << ")\n";
+      out.write(seq.data() + at, (std::streamsize)(r.end - r.start)) << '\n';
+      at += r.end - r.start;
+    }
+  }
+  if (o.verbose || o.statistics) std::cout << dna::size() << ',' << regions.size() << ',' << written << '\n';
+  return 0;
+}
+
 static int decompress(const Options& o) {
+  if (!o.regions.empty()) return extract(o);
   std::ifstream in{o.input, std::ios::binary};
   shared_tree tree = shared_tree::deserialize(in);
   const std::size_t width = tree.width();

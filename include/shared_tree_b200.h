@@ -120,6 +120,21 @@ int stb_decode_leaves(const stb_tree* tree, uint64_t first, uint64_t count, uint
 int stb_decode_ascii(const stb_tree* tree, uint64_t first, uint64_t count, char* out, int memory);
 /* operator[] (src/shared_tree.cpp:268-291), batched: out[i] = tree[index[i]] */
 int stb_random_access(const stb_tree* tree, const uint64_t* index, uint64_t queries, uint64_t* out, int memory);
+/* Bases [start[i], end[i]) of the decoded sequence, 0-based and half-open as in BED.
+ * Base b is nucleotide b % dna_size of leaf b / dna_size; valid ends are <= width() * dna_size.
+ * strand[i]: 0 = as stored, 1 = reverse complement (dna::inverted, src/dna.cpp).
+ * strand may be NULL, meaning all regions are forward.
+ * Letters as stb_decode_ascii spells them.  Regions go back to back in input order:
+ * region i starts at out[sum of the lengths of regions 0..i-1].
+ * *written receives the total length.
+ * start, end, strand and out all live in `memory` (device start and end: 8-byte aligned).
+ * out == NULL: only *written is set.
+ * cap < total: STB_ERR_BUFFER_TOO_SMALL, *written = total, out untouched.
+ * Regions may overlap, come in any order, be empty or span the whole sequence.  Every region is checked
+ * before anything is written: start > end, or a strand outside {0, 1}: STB_ERR_INVALID_ARG; end past the
+ * sequence: STB_ERR_OUT_OF_RANGE.  n_regions == 0: STB_OK with *written = 0. */
+int stb_extract_regions(const stb_tree* tree, const uint64_t* start, const uint64_t* end, const uint8_t* strand,
+                        uint64_t n_regions, char* out, uint64_t cap, int memory, uint64_t* written);
 
 /* ---- value primitives (no device needed) ------------------------------------------------
  * The very functions the kernels run (__host__ __device__), callable on the host so that the
