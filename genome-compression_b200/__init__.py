@@ -258,8 +258,16 @@ class SharedTree:
         self._check(lib.stb_copy_layer(self._h, k, out.ctypes.data, out.shape[0], HOST))
         return out
 
-    def histogram(self, k: int) -> np.ndarray:
+    def histogram(self, k: int, out=None):
+        """References from node layer k into its child layer.  out: a contiguous int64 or uint64 CUDA tensor of at
+        least that many elements, filled on the device."""
         n = self.leaf_count() if k == 0 else self.layer_count(k - 1)
+        if out is not None:
+            import torch
+            if not (_is_device_tensor(out) and out.is_contiguous() and out.dtype in (torch.int64, torch.uint64)):
+                raise TypeError("histogram(out=...): a contiguous CUDA tensor of torch.int64 or torch.uint64")
+            self._check(lib.stb_histogram(self._h, k, out.data_ptr(), out.numel(), DEVICE))
+            return out
         out = np.zeros(n, dtype=np.uint64)
         self._check(lib.stb_histogram(self._h, k, out.ctypes.data, n, HOST))
         return out

@@ -447,6 +447,8 @@ extract_regions_kernel(const unsigned long long* __restrict__ start, const unsig
 
 // width() for a tree that was not built here: nulls exist only on the logical right
 // edge, so walk that edge: a present second child means the first subtree is full.
+// A node whose children are both null is never followed: *out = WIDTH_NULL_WALK instead.
+constexpr unsigned long long WIDTH_NULL_WALK = ~0ull;
 __global__ void width_kernel(LayerPtrs layers, int n_layers, uint32_t root, unsigned long long* __restrict__ out) {
   if (threadIdx.x || blockIdx.x) return;
   unsigned long long w = 0;
@@ -463,6 +465,12 @@ __global__ void width_kernel(LayerPtrs layers, int n_layers, uint32_t root, unsi
       w += 1ull << layer;
       cur = compose(second, m, t);
     } else {
+      // tested before composing: under a mirrored parent compose() sets the mirror bit of a null
+      // (a stream's null carries no invariant bit), and ptr_is_null would no longer see it
+      if (ptr_is_null(first)) {
+        *out = WIDTH_NULL_WALK;
+        return;
+      }
       cur = compose(first, m, t);
     }
   }
@@ -490,6 +498,7 @@ int compute_width(Tree& t) {
   STB_CUDA(t, cudaMemcpyAsync(&w, d.ptr, 8, cudaMemcpyDeviceToHost, t.stream));
   STB_CUDA(t, cudaStreamSynchronize(t.stream));
   STB_CUDA(t, cudaGetLastError());
+  if (w == WIDTH_NULL_WALK) return t.fail(STB_ERR_BAD_STREAM, "a node on the right edge has no child: both are null");
   t.width = w;
   return STB_OK;
 }

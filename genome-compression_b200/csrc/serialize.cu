@@ -389,7 +389,15 @@ __device__ __forceinline__ uint32_t ptr_decode(uint32_t b0, uint32_t rest /* the
   return idx | (((b0 >> 4) & 1u) << 29) | (((b0 >> 5) & 1u) << 30);
 }
 
-// result[0] = absolute offset of the byte after the layer's last pointer, result[1] = 1 when a pointer indexes past `below`
+// A decoded child pointer the tree cannot follow: an index past the layer below, or the null index with the
+// mirror or transpose bit set (ptr_is_null does not count that as null, so it would be followed to index 2^29-1).
+__host__ __device__ __forceinline__ bool ptr_unfollowable(uint32_t raw, uint32_t below) {
+  const uint32_t idx = raw & IDX_MASK;
+  return idx == IDX_MASK ? (raw & (MIRROR | TRANSPOSE)) != 0u : idx >= below;
+}
+
+// result[0] = absolute offset of the byte after the layer's last pointer, result[1] = 1 when a pointer cannot be
+// followed (ptr_unfollowable)
 __global__ void __launch_bounds__(DP_THREADS)
 parse_emit_kernel(const uint8_t* __restrict__ stream, uint64_t begin, uint32_t start_off, const uint2* __restrict__ tile_entry,
                   uint32_t* __restrict__ out, uint32_t n_ptrs, uint32_t below, unsigned long long* __restrict__ result) {
@@ -421,8 +429,7 @@ parse_emit_kernel(const uint8_t* __restrict__ stream, uint64_t begin, uint32_t s
     const uint32_t number = entry.y + local;  // < 2^32: entry.y < n_ptrs <= 2^30, local <= 8192
     pos += seg + 1u;
     if (number < n_ptrs) {
-      const uint32_t idx = raw & IDX_MASK;
-      bad |= idx != IDX_MASK && idx >= below;
+      bad |= ptr_unfollowable(raw, below);
       sout[local] = raw;
       if (number == n_ptrs - 1u) result[0] = tile_begin + (uint64_t)t * DP_CHUNK + pos;
     }
@@ -448,8 +455,14 @@ parse_leaves_kernel(const uint8_t* __restrict__ stream, uint64_t begin, uint32_t
 // shared_tree::deserialize, src/shared_tree.cpp:520-538; pointers come back with invariant = false (:162).
 // The stream is copied to the device once; the layers are parsed there (see above), the small top of the
 // tree on the host.  A foreign or damaged stream must not make the device follow wild indices (an illegal
-// address is sticky for the whole process): every non-null child index has to exist in the layer below, the
-// root in the top layer.  The reference trusts its input.
+// address is sticky for the whole process).  The reference trusts its input; here STB_ERR_BAD_STREAM rejects:
+//   - a stream that ends inside the header, the leaf table or a node;
+//   - no leaves, a node layer of no nodes, or no node layer at all;
+//   - a leaf table or a layer too large for the pointer format to index;
+//   - a child pointer that indexes past the layer below, or the null index with the mirror or transpose bit set;
+//   - a root that does not index the top layer (a null root included);
+//   - a right edge that leads into a null: the node the width walk reaches has no child to go on with
+//     (compute_width).  Nulls elsewhere are read as they are; builds write them nowhere else.
 int deserialize_tree(Tree& t, const uint8_t* in, uint64_t len) {
   static const uint32_t start[4] = {0u, 16u, 4112u, 1052688u};
   t.clear();
@@ -480,6 +493,7 @@ int deserialize_tree(Tree& t, const uint8_t* in, uint64_t len) {
   const int leaf_bytes = (t.S + 1) / 2;
   if (n_leaves > (len - o) / (uint64_t)leaf_bytes) return t.fail(STB_ERR_BAD_STREAM, "stream ends inside the leaf table");
   if (n_leaves >= IDX_MASK) return t.fail(STB_ERR_BAD_STREAM, "leaf table larger than the pointer format can index");
+  if (n_leaves == 0) return t.fail(STB_ERR_BAD_STREAM, "stream holds no leaves");
 
   // the whole stream on the device (the handle's grow-only staging buffer), zero-padded by one tile
   const uint64_t padded = ((len + 31) & ~31ull) + DP_TILE + 64;
@@ -530,6 +544,7 @@ int deserialize_tree(Tree& t, const uint8_t* in, uint64_t len) {
     if (count > (len - o) / 2) return bad("layer size exceeds the remaining stream");
     if (count >= IDX_MASK) return bad("layer larger than the pointer format can index");
     const size_t k = t.layers.size();
+    if (count == 0) return bad("node layer " + std::to_string(k) + " holds no nodes");
     t.layers.emplace_back();
     Layer& layer = t.layers.back();
     layer.count = count;
@@ -539,9 +554,8 @@ int deserialize_tree(Tree& t, const uint8_t* in, uint64_t len) {
       for (uint64_t i = 0; i < count; ++i) {
         uint2 nd;
         if (!read_ptr(nd.x) || !read_ptr(nd.y)) return bad("stream ends inside a node");
-        const uint32_t l = nd.x & IDX_MASK, r = nd.y & IDX_MASK;
-        if ((l != IDX_MASK && l >= below) || (r != IDX_MASK && r >= below))
-          return bad("a node of layer " + std::to_string(k) + " points past the end of the layer below");
+        if (ptr_unfollowable(nd.x, (uint32_t)below) || ptr_unfollowable(nd.y, (uint32_t)below))
+          return bad("a node of layer " + std::to_string(k) + " points past the end of the layer below or holds a flagged null");
         nodes[i] = nd;
       }
       STB_CUDA(t, cudaMemcpyAsync(layer.nodes.ptr, nodes.data(), count * sizeof(uint2), cudaMemcpyHostToDevice, st));
@@ -573,7 +587,7 @@ int deserialize_tree(Tree& t, const uint8_t* in, uint64_t len) {
       STB_CUDA(t, cudaStreamSynchronize(st));
       STB_CUDA(t, cudaGetLastError());
       if (res[0] == 0 || res[0] > len) return bad("stream ends inside a node");
-      if (res[1]) return bad("a node of layer " + std::to_string(k) + " points past the end of the layer below");
+      if (res[1]) return bad("a node of layer " + std::to_string(k) + " points past the end of the layer below or holds a flagged null");
       o = res[0];
     }
     below = count;

@@ -110,7 +110,12 @@ int stb_sort_tree(stb_tree* tree);
 /* ---- .dag stream: src/shared_tree.cpp:488-546 ----------------------------------- */
 int stb_bytes(const stb_tree* tree, uint64_t* out);                      /* bytes() */
 int stb_serialize(const stb_tree* tree, uint8_t* out, uint64_t cap, int memory, uint64_t* written);
-int stb_deserialize(stb_tree* tree, const uint8_t* bytes, uint64_t len); /* host bytes */
+/* deserialize from host bytes.  STB_ERR_BAD_STREAM for: a stream that ends inside the header, the leaf table or a
+ * node; no leaves, a node layer of no nodes, or no node layer; a leaf table or layer too large for the pointer format;
+ * a child pointer past the end of the layer below, or the null index (segment 3, offset 0xfffffff) with the mirror or
+ * transpose bit set; a root that does not index the top layer; a node on the logical right edge whose children are
+ * both null.  Nulls elsewhere are accepted (builds never write them; width() and decode assume there are none). */
+int stb_deserialize(stb_tree* tree, const uint8_t* bytes, uint64_t len);
 
 /* ---- decode ------------------------------------------------------------------------ */
 /* shared_tree::iterator (src/shared_tree.cpp:553-614): leaves first..first+count-1
