@@ -136,7 +136,9 @@ leaf_insert_text_kernel(const char* __restrict__ body, uint64_t n_leaves, int S_
       if (bad != 0xFFFFFFFFu) {
         uint32_t c = tile[bad];
         if (c >= 'a' && c <= 'z') c -= 32;
-        atomicMin(&flags->bad_symbol, ((tile_first * S + bad) << 8) | c);
+        // `body` starts at leaf pos0 of the text: offsets count from the text's start, so that the smallest one is
+        // the first bad byte even when the text is inserted in several launches (the streaming build)
+        atomicMin(&flags->bad_symbol, (((uint64_t)pos0 * S + tile_first * S + bad) << 8) | c);
       }
       insert_leaf<DIRECT>(v, S, pos0 + (uint32_t)(tile_first + j), tab, tmp + tile_first + j, flags);
     }
@@ -182,8 +184,9 @@ __device__ __forceinline__ bool acgt12_leaf(const uint8_t* smem, const uint8_t* 
     if (bad != 0xFFFFFFFFu) {
       uint32_t ch = tile[bad];
       if (ch >= 'a' && ch <= 'z') ch -= 32;
-      // (a lookup launch starts at leaf pos0 of the body its caller holds: offsets count from the body's start)
-      const uint64_t text0 = LOOKUP ? (uint64_t)pos0 * 12 : 0;
+      // (every launch starts at leaf pos0 of the text: a lookup launch, and every chunk of the streaming build;
+      // offsets count from the text's start)
+      const uint64_t text0 = (uint64_t)pos0 * 12;
       atomicMin(&flags->bad_symbol, ((text0 + tile_first * 12 + bad) << 8) | ch);
     }
     const unsigned long long canon = canonical_leaf(v, 12, f4);
